@@ -2,6 +2,7 @@
 """bench.py -- throughput of the greedy hot path on BASELINE.json's configs.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--config 2|3|4|5] [--seqs S] [--impl ours|reference]
+                    [--dump-outputs DIR]
 
 --config 2 (default, the configuration the metric is quoted on): 1 M synthetic random RNAs U{60..200} per GPU,
             `byseq pl=1 c=fastest.conf`; weak scaling (S per GPU, ranks take disjoint batches).
@@ -25,6 +26,8 @@ Printed by rank 0 as ONE JSON line:
   cpu_baseline  the UNMODIFIED Python reference (baseline/_ref/SQUARNA, `byseq t=<cores>`) on a bounded sample of
            the same workload, and the plain-C oracle port beside it
 `--impl reference` times only the CPU side: the Python reference through its own Predict() (rank 0; other ranks exit).
+`--dump-outputs DIR` writes, after the timed steps, what the timed path returned in its last step (rank 0's share) as
+float32 / float64 .npy files, at most 64 MB in all (see dump_outputs); the inputs are a pure function of the arguments.
 """
 import argparse
 import io
@@ -304,6 +307,45 @@ def load_traffic(kernel):
     return None
 
 
+DUMP_BYTES = 64 * 10 ** 6
+
+
+def dump_outputs(dirname, n, rows=None, ragged=None, ids=None):
+    """--dump-outputs: what the timed path returned for its n output items, as DIR/<name>.npy, so that two builds can be
+    compared output for output.  rows: name -> array whose first axis runs over the items; ragged: name -> (offsets,
+    values), item k's values at values[offsets[k]:offsets[k + 1]] (written as <name>.npy + <name>_offsets.npy).  float64
+    arrays stay float64, one- and two-byte codes become float32, wider integers float64.  When everything does not fit
+    in 64 MB, items are taken in a fixed seeded order until the budget is spent.  item_index.npy lists the kept items, as
+    positions in the workload's input order when `ids` maps each item to one."""
+    from squarna_b200.sharding import take_csr
+
+    def out_size(dt):
+        return 4 if np.dtype(dt).itemsize <= 2 and np.dtype(dt).kind != "f" else 8
+
+    def as_float(a):
+        return np.asarray(a, dtype=np.float32 if out_size(a.dtype) == 4 else np.float64)
+
+    rows = {k: np.asarray(v) for k, v in (rows or {}).items()}
+    ragged = {k: (np.asarray(o, dtype=np.int64), np.asarray(v)) for k, (o, v) in (ragged or {}).items()}
+    per_item = np.full(n, 8, dtype=np.int64)                                       # item_index
+    for v in rows.values():
+        per_item += v.size // max(n, 1) * out_size(v.dtype)
+    for o, v in ragged.values():
+        per_item += np.diff(o) * out_size(v.dtype) + 8
+    order = np.random.default_rng(SEED).permutation(n)
+    budget = DUMP_BYTES - 256 * (1 + len(rows) + 2 * len(ragged))                 # (.npy headers)
+    keep = np.sort(order[np.cumsum(per_item[order]) <= budget])
+    os.makedirs(dirname, exist_ok=True)
+    np.save(os.path.join(dirname, "item_index.npy"), (keep if ids is None else np.asarray(ids)[keep]).astype(np.float64))
+    for name, v in rows.items():
+        np.save(os.path.join(dirname, name + ".npy"), as_float(v[keep]))
+    for name, (o, v) in ragged.items():
+        sub, sub_off = take_csr(v, o, keep)
+        np.save(os.path.join(dirname, name + ".npy"), as_float(sub))
+        np.save(os.path.join(dirname, name + "_offsets.npy"), sub_off.astype(np.float64))
+    return len(keep)
+
+
 # ------------------------------------------------------------------------------ configs 2 and 5: the fast lane
 def bench_fast(args, rank, world, local):
     import torch
@@ -465,6 +507,12 @@ def bench_fast(args, rank, world, local):
         keep = (dfl & 8) == 0
         assert np.array_equal(dp_milli.cpu().numpy().reshape(-1, 2)[keep], pm[keep])
         assert np.array_equal(dp_ns.cpu().numpy().view(np.uint16), p_ns.numpy().view(np.uint16))
+
+    # the device leg's last step in the byte format (the other legs were checked equal to it above): raw scores,
+    # ASCII dot-brackets, stem counts of this rank's batch
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, n, rows={"scores": dsc.reshape(n, 3), "n_stems": d_ns.cpu().numpy()},
+                     ragged={"dbn": (off, d_dbn.cpu().numpy())}, ids=idx if strong else None)
 
     # strong scaling: finished results gathered on rank 0 in input order (host-side, after the timed region)
     gathered = None
@@ -662,6 +710,26 @@ def bench_config3(args, rank, world, local):
             structs += sum(len(r[1]) for r in results[c])
     barrier()
     e2e_s = (time.perf_counter() - t0) / args.steps
+    if args.dump_outputs and rank == 0:
+        # the last predict_many of every length class, back in this rank's entry order: consensus, the structures of
+        # each entry back to back, their three scores each
+        preds = [None] * len(mine)
+        for c in groups:
+            for k, r in zip([k for k, e in enumerate(mine) if workloads.config3_conf(len(e[0])) == c], results[c]):
+                preds[k] = r
+
+        def offsets(parts):
+            o = np.zeros(len(parts) + 1, dtype=np.int64)
+            np.cumsum([len(p) for p in parts], out=o[1:])
+            return o
+
+        cons = [p[0].encode() for p in preds]
+        dbns = [b"".join(s[0].encode() for s in p[1]) for p in preds]
+        scores = [[float(x) for s in p[1] for x in s[1]] for p in preds]
+        dump_outputs(args.dump_outputs, len(mine), rows={"n_structures": np.array([len(p[1]) for p in preds])},
+                     ragged={"consensus": (offsets(cons), np.frombuffer(b"".join(cons), np.uint8)),
+                             "structures": (offsets(dbns), np.frombuffer(b"".join(dbns), np.uint8)),
+                             "scores": (offsets(scores), np.array([x for s in scores for x in s], np.float64))}, ids=idx)
     # value leg: the C-ABI batch call alone on prepared batches (no Python preparation / result assembly)
     batches = []
     for c, es in groups.items():
@@ -784,8 +852,8 @@ def bench_config4(args, rank, world, local):
         mat, cells = A._yield_many(entries, first["bpweights"], False, first["minlen"], first["minbpscore"], device=local, matrix=(L, thr))
         dbn = A.MatrixToDBNs(mat, first["minbpscore"], n_rows, cells=cells)[0]
         ent2 = [(r, None, dbn) for r in rows]
-        A._yield_many(ent2, first["bpweights"], False, first["minlen"], first["minbpscore"], device=local, matrix=(L, thr))
-        return dbn
+        mat2, cells2 = A._yield_many(ent2, first["bpweights"], False, first["minlen"], first["minbpscore"], device=local, matrix=(L, thr))
+        return dbn, mat2, cells2
 
     for _ in range(max(args.warmup, 3)):
         dbn1 = step1()
@@ -795,11 +863,17 @@ def bench_config4(args, rank, world, local):
     t0 = time.perf_counter()
     kms, launches = 0.0, 0
     for _ in range(args.steps):
-        step1()
+        dbn, mat, cells = step1()
         st = ctx.stats()
         kms += st["kernel_ms"]; launches += st["launches"]
     torch.cuda.synchronize()
     step1_s = (time.perf_counter() - t0) / args.steps
+    if args.dump_outputs:
+        # one item, the alignment: the first iteration's structure, the second iteration's stem matrix and the cells
+        # MatrixToDBNs would walk (empty when there are too many for the device ranking)
+        cells = np.zeros(0, np.int32) if cells is None else cells
+        dump_outputs(args.dump_outputs, 1, rows={"stem_matrix": mat[None]},
+                     ragged={"dbn": ([0, L], np.frombuffer(dbn.encode(), np.uint8)), "cells": ([0, len(cells)], cells)})
     with tempfile.TemporaryDirectory() as tmp:
         path = os.path.join(tmp, "c4.afa")
         with open(path, "w") as f:
@@ -852,9 +926,15 @@ def main():
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg (profiling runs)")
     ap.add_argument("--no-cli", action="store_true", help="skip the CLI-level end-to-end leg of config 2")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the timed path returned in its last step as DIR/<name>.npy")
     args = ap.parse_args()
     if args.steps is None:
         args.steps = {2: 20, 5: 3, 3: 1, 4: 3}[args.config]
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes this project's outputs; the reference arm has none")
     if args.seqs is None:
         args.seqs = {2: 1_000_000, 5: 10_000, 3: 100_000 if args.gpus >= 8 else 20_000, 4: 2000}[args.config]
     rank = int(os.environ.get("RANK", "0"))

@@ -19,8 +19,12 @@ def build():
             os.path.join(_ROOT, "squarna_b200", "csrc", "sqrn_params.h")]
     if not os.path.exists(_SO) or any(os.path.getmtime(s) > os.path.getmtime(_SO) for s in srcs):
         os.makedirs(os.path.dirname(_SO), exist_ok=True)
+        # parallel test workers may all build: each writes its own file and renames it into place, so that no
+        # worker loads a library another one is still writing
+        tmp = "%s.%d.tmp" % (_SO, os.getpid())
         subprocess.check_call(["g++", "-O2", "-g", "-std=c++17", "-ffp-contract=off", "-fPIC", "-shared",
-                               "-Wno-unknown-pragmas", "-o", _SO, srcs[0], "-lm"])
+                               "-Wno-unknown-pragmas", "-o", tmp, srcs[0], "-lm"])
+        os.replace(tmp, _SO)
     return _SO
 
 

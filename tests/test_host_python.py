@@ -460,6 +460,37 @@ def test_bench_helpers_without_a_gpu(monkeypatch):
     assert bench.bind_near_gpu(0) is None
 
 
+def test_bench_dump_outputs_format_budget_and_sample(tmp_path, monkeypatch):
+    """bench.py --dump-outputs: float32 / float64 .npy files within the byte budget, a sample of whole items that is
+    the same from run to run, and each kept item's values equal to the input arrays'"""
+    import numpy as np
+    import bench
+    rng = np.random.default_rng(1)
+    n = 3000
+    off = np.zeros(n + 1, np.int64)
+    np.cumsum(rng.integers(60, 201, n), out=off[1:])
+    dbn = rng.choice(np.frombuffer(b".()[]", np.uint8), int(off[-1]))
+    sc, ns = rng.random((n, 3)), rng.integers(0, 40, n).astype(np.int32)
+    kw = dict(rows={"scores": sc, "n_stems": ns}, ragged={"dbn": (off, dbn)})
+    assert bench.dump_outputs(str(tmp_path / "all"), n, **kw) == n
+    monkeypatch.setattr(bench, "DUMP_BYTES", 100_000)
+    k = bench.dump_outputs(str(tmp_path / "a"), n, **kw)
+    assert 0 < k < n and bench.dump_outputs(str(tmp_path / "b"), n, **kw) == k
+    files = sorted(os.listdir(tmp_path / "a"))
+    assert files == ["dbn.npy", "dbn_offsets.npy", "item_index.npy", "n_stems.npy", "scores.npy"]
+    assert sum(os.path.getsize(tmp_path / "a" / f) for f in files) <= 100_000
+    got = {f[:-4]: np.load(tmp_path / "a" / f) for f in files}
+    for f in files:
+        assert got[f[:-4]].dtype in (np.float32, np.float64)
+        assert np.array_equal(got[f[:-4]], np.load(tmp_path / "b" / f))
+    idx = got["item_index"].astype(np.int64)
+    assert len(idx) == k and (np.diff(idx) > 0).all()
+    assert np.array_equal(got["scores"], sc[idx]) and np.array_equal(got["n_stems"], ns[idx])
+    o = got["dbn_offsets"].astype(np.int64)
+    for j, b in enumerate(idx.tolist()):
+        assert np.array_equal(got["dbn"][o[j]:o[j + 1]], dbn[off[b]:off[b + 1]])
+
+
 def test_sqrndbnseq_host_python_on_the_reference_cases(monkeypatch):
     """squarna_b200.SQRNdbnseq.SQRNdbnseq -- _prepare (gaps, separators, restraints, reactivity decoding), the result
     assembly (level codes -> glyphs, ReAlign, separators, paramset lists, int-0 score) -- on the end-to-end cases of
