@@ -186,6 +186,25 @@ SQRN_API int  sqrn_yield_stems_batch(sqrn_ctx *ctx, const sqrn_paramset *ps,
 SQRN_API int  sqrn_stem_matrix_batch(sqrn_ctx *ctx, const sqrn_paramset *ps, const sqrn_batch *in, double *matrix,
                             double threshold, int64_t cap_cells, int64_t *n_cells, int32_t *cells);
 
+/* The Nussinov builder (SQRNalgos.py: Nussinov + BackTrack, what RunAlgo runs for algorithm "N") for a batch, on the
+ * device: per sequence the minimum-energy nested structure over the pairs of its stems, energy of a pair = -(score of
+ * its stem), followed back from (0, N-1) with the hairpin rule `minloop` and the separators ';' '&' of `symbols`.
+ * Host buffers in and out.
+ *   offsets      [n_seqs+1], offsets[0] == 0; symbols [offsets[n_seqs]]: the ungapped sequences (N <= SQRN_MAX_LEN);
+ *   stem_offsets [n_seqs+1], stems [3 * ...] (i, j, len), scores [...]: as sqrn_yield_stems_batch returns them; a stem
+ *                holds the pairs (i+t, j-t), t < len; a pair two stems hold takes the later stem's score;
+ *   minloop      >= 0 (RunAlgo passes 3);
+ *   pair_offsets [n_seqs+1] out; pairs [2 * sum_b floor(N_b / 2)] int32 out: sequence b's pairs (v, w), sorted, at
+ *                pairs + 2 * pair_offsets[b] (a sequence has at most N/2 pairs, so this size always suffices).
+ * SQRN_E_BADARG: a stem outside [0, N) or with len < 1, a sequence longer than SQRN_MAX_LEN, minloop < 0.
+ * Sequences of up to ~238 positions (the opt-in shared memory of a B200) keep their DP triangle in shared memory, longer
+ * ones in a device workspace of at most 4 GiB (at least one 1.28 GB slot at 16 000 nt), which the context keeps at the
+ * size of its largest call until sqrn_ctx_destroy; one CTA per sequence either way, longest first, the two tiers run
+ * concurrently.                                                                                                      */
+SQRN_API int  sqrn_nussinov_batch(sqrn_ctx *ctx, int64_t n_seqs, const int64_t *offsets, const uint8_t *symbols,
+                                  const int64_t *stem_offsets, const int32_t *stems, const double *scores,
+                                  int32_t minloop, int64_t *pair_offsets, int32_t *pairs);
+
 /* ---- single-path fast lane (poollim == 1: `byseq pl=1`, SQUARNA.py:887-935) --
  * One parameter set, default reactivities, no restraints: one structure per
  * sequence, written as ASCII dot-bracket.  `symbols`/`offsets`/outputs are HOST

@@ -621,12 +621,15 @@ def _cell_scorer(p, paramset, smat, bpp_mode=0, bpp_term=None):
     return score
 
 
-def RunAlgo(seq, stems, cell_score, minlen, minscore, algo="E", levellimit=3):
+def RunAlgo(seq, stems, cell_score, minlen, minscore, algo="E", levellimit=3, pairs=None):
     """one non-greedy prediction (seq.py:548-595).  stems: AnnotateStems output [[pairs, len, score], ...];
-    cell_score(v, w) = bpscorematrix[v, w]."""
+    cell_score(v, w) = bpscorematrix[v, w].  pairs: what the builder returned when it ran elsewhere (the device
+    Nussinov builder); `stems` is then not read."""
     from . import SQRNalgos
     N = len(seq)
-    if algo == "E":
+    if pairs is not None:
+        pass                                         # the builder already ran
+    elif algo == "E":
         pairs = SQRNalgos.Edmonds(stems)
     elif algo == "N":
         pairs = SQRNalgos.Nussinov(seq, stems, N, SEPS)
@@ -678,13 +681,20 @@ def _predict_many_mixed(entries, paramsets, conslim, toplim, hardrest, rankbydif
             others = [a for a in use if a != "G"]             # set order, as in the reference's `for algo in algos`
             if others:
                 batch = _make_batch(preps, idx, comp, stemmatrix, interchainonly, bpp=bpp)
-                for q, (k, (st, sc)) in enumerate(zip(idx, ctx.yield_stems(ps, batch))):
+                found = ctx.yield_stems(ps, batch)
+                # Nussinov on the device when the context has the builder (the host SQRNalgos.Nussinov otherwise): one
+                # call for the group, over the stems just enumerated; the stem lists are built only for E / H
+                nuss = getattr(ctx, "nussinov", None) if "N" in others else None
+                dev_pairs = nuss(batch.symbols, batch.offsets, found, minloop=3) if nuss is not None else None
+                lists = dev_pairs is None or any(a != "N" for a in others)
+                for q, (k, (st, sc)) in enumerate(zip(idx, found)):
                     p = preps[k]
-                    stems = [[[(i + t, j - t) for t in range(ln)], ln, float(s_)] for (i, j, ln), s_ in zip(st.tolist(), sc.tolist())]
+                    stems = [[[(i + t, j - t) for t in range(ln)], ln, float(s_)] for (i, j, ln), s_ in zip(st.tolist(), sc.tolist())] if lists else None
                     cell = _cell_scorer(p, ps, smat_np, bpp[0] if bpp else 0, bpp[1][q] if bpp else None)
                     ll = levellimit if levellimit is not None else 3 - int(len(p.shortseq) > 500)
                     for algo in others:
-                        stemset = RunAlgo(p.shortseq, stems, cell, ps["minlen"], ps["minbpscore"], algo, ll)
+                        pairs = dev_pairs[q].tolist() if algo == "N" and dev_pairs is not None else None
+                        stemset = RunAlgo(p.shortseq, stems, cell, ps["minlen"], ps["minbpscore"], algo, ll, pairs=pairs)
                         per_ps[k][psi].append((stemset, ScoreStruct(p.shortseq, stemset, p.shortreacts)))
             if "G" in use:
                 batch = _make_batch(preps, idx, comp, stemmatrix, interchainonly, bpp=bpp, hardrest=False,

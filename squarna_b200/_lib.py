@@ -22,7 +22,8 @@ EXPORTS = ["sqrn_abi_version", "sqrn_device_count", "sqrn_ctx_create", "sqrn_ctx
            "sqrn_fast_predict_host", "sqrn_fast_predict_device", "sqrn_ctx_last_stats", "sqrn_debug_run",
            "sqrn_ctx_set_tuning", "sqrn_text_parse", "sqrn_text_ungap", "sqrn_text_format",
            "sqrn_fast_predict_packed_host", "sqrn_pack_symbols", "sqrn_unpack_dbn", "sqrn_fast_last_flags",
-           "sqrn_stem_matrix_batch", "sqrn_fast_predict_packed_device", "sqrn_codes_to_ascii", "sqrn_dbn_pairs"]
+           "sqrn_stem_matrix_batch", "sqrn_fast_predict_packed_device", "sqrn_codes_to_ascii", "sqrn_dbn_pairs",
+           "sqrn_nussinov_batch"]
 
 _lib = None
 
@@ -62,6 +63,7 @@ def load():
     L.sqrn_dbn_pairs.argtypes = [i64, vp, C.c_int32, vp, vp, vp, C.POINTER(C.c_int64)]
     L.sqrn_fast_last_flags.argtypes = [vp, i64, vp]
     L.sqrn_stem_matrix_batch.argtypes = [vp, C.POINTER(ParamSet), C.POINTER(Batch), vp, C.c_double, i64, C.POINTER(i64), vp]
+    L.sqrn_nussinov_batch.argtypes = [vp, i64, vp, vp, vp, vp, vp, i32, vp, vp]
     L.sqrn_ctx_last_stats.argtypes = [vp, C.POINTER(i64), C.POINTER(C.c_double), C.POINTER(i64)]
     L.sqrn_debug_run.argtypes = [vp, C.POINTER(ParamSet), C.POINTER(Batch), C.c_int, C.c_int] + [vp] * 11 + [C.c_int]
     L.sqrn_text_parse.argtypes = [vp, i64, C.c_int, C.POINTER(i64), C.POINTER(i64), i64, i64, vp, vp, vp, vp]
@@ -527,6 +529,24 @@ class Context:
             self._check(rc)
             break
         return [(st[off[b]:off[b + 1]].copy(), sc[off[b]:off[b + 1]].copy()) for b in range(n)]
+
+    def nussinov(self, symbols, offsets, stems, minloop=3):
+        """the Nussinov builder (SQRNalgos.Nussinov + BackTrack) on the device for a batch (include/sqrn.h:
+        sqrn_nussinov_batch).  symbols / offsets: the ungapped sequences as in PackedBatch; stems: per sequence
+        (stems (k,3) int32, scores (k,) float64), as yield_stems returns them.  Returns per sequence its base pairs as
+        an (n, 2) int32 array sorted by (v, w)."""
+        offsets = np.ascontiguousarray(offsets, np.int64)
+        symbols = np.ascontiguousarray(symbols, np.uint8)
+        n = len(offsets) - 1
+        so = np.zeros(n + 1, np.int64)
+        np.cumsum([len(sc) for _, sc in stems], out=so[1:])
+        st = np.concatenate([np.asarray(x, np.int32).reshape(-1, 3) for x, _ in stems] + [np.zeros((1, 3), np.int32)])
+        sc = np.concatenate([np.asarray(x, np.float64).ravel() for _, x in stems] + [np.zeros(1)])
+        po = np.zeros(n + 1, np.int64)
+        pairs = np.zeros((max(int((np.diff(offsets) // 2).sum()), 1), 2), np.int32)
+        self._check(self.L.sqrn_nussinov_batch(self.h, n, ptr(offsets), ptr(symbols), ptr(so), ptr(st), ptr(sc),
+                                               int(minloop), ptr(po), ptr(pairs)))
+        return [pairs[po[b]:po[b + 1]] for b in range(n)]
 
     def stem_matrix(self, paramset, batch, threshold, cap_cells=65536):
         """alignment step 1 on the device (include/sqrn.h): batch carries cols and smat_L = alignment length (no smat).

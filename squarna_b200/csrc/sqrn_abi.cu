@@ -18,6 +18,7 @@
 #include <unordered_map>
 #include <vector>
 #include "sqrn_params.h"
+#include "sqrn_nussinov.cuh"
 
 using namespace sqrn;
 
@@ -194,7 +195,8 @@ struct CachedStems {
 
 enum { B_OFF, B_OFF32, B_SYM, B_RCODE, B_RVALS, B_RFPOS, B_RFNEG, B_RCLASS, B_RBOFF, B_RB, B_SMAT, B_COLS, B_BPP, B_BPPOFF,
        W_ORDER, W_ISEQ, W_IOFF, W_ISTEMS, W_SUBOPT, W_COUNTER, W_OOFF, W_OSTEMS, W_ON, W_OFIN, W_ORAW,
-       W_OFLAGS, W_DOFF, W_DBNA, W_DBNC, W_NCALLS, W_OVF, W_GENT, W_GBPS, W_GQB, W_GCNT, W_GCNT2, W_GSTAT, W_OVF2, W_RNDC, W_RNDL, W_BASE, W_BASEOFF, W_BASEN, W_BASEBEND, W_MAT, W_CELLCNT, W_CELLS, W_CELLS2, NBUF };
+       W_OFLAGS, W_DOFF, W_DBNA, W_DBNC, W_NCALLS, W_OVF, W_GENT, W_GBPS, W_GQB, W_GCNT, W_GCNT2, W_GSTAT, W_OVF2, W_RNDC, W_RNDL, W_BASE, W_BASEOFF, W_BASEN, W_BASEBEND, W_MAT, W_CELLCNT, W_CELLS, W_CELLS2,
+       NU_COLPTR, NU_PK, NU_PE, NU_ORDER, NU_OUTBASE, NU_OUTP, NU_OUTN, NU_CNT, NBUF };
 
 // ------------------------------------------------------------- launch plan
 struct Plan { int tw, threads, tpc, grid; size_t smem; Layout L; int fast_ncap = 0; int cluster = 0; bool cl_plain = false;
@@ -224,6 +226,7 @@ struct sqrn_ctx {
     int no_glist = 0;            // tuning knob: CTA teams rescan every step (no global persistent list)
     int gl_rebuild = 0;          // tuning knob: rebuild period of the binned global list in passes (0: the default)
     CachedResult cres; CachedStems cstems;
+    void *nu_ws = nullptr; size_t nu_ws_bytes = 0;   // workspace of sqrn_nussinov_batch (exact size, grown on demand)
 };
 
 static std::string g_create_err;
@@ -309,6 +312,7 @@ extern "C" void sqrn_ctx_destroy(sqrn_ctx *ctx)
     for (int c = 0; c < FAST_MAX_CHUNKS; c++) { cudaEventDestroy(ctx->ev_in[c]); cudaEventDestroy(ctx->ev_k0[c]); cudaEventDestroy(ctx->ev_k1[c]); cudaEventDestroy(ctx->ev_o[c]); cudaEventDestroy(ctx->ev_l0[c]); cudaEventDestroy(ctx->ev_l1[c]); }
     if (ctx->hflags) cudaFreeHost(ctx->hflags);
     if (ctx->horder) cudaFreeHost(ctx->horder);
+    if (ctx->nu_ws) cudaFree(ctx->nu_ws);
     delete ctx;
 }
 
@@ -2088,4 +2092,211 @@ extern "C" int sqrn_debug_run(sqrn_ctx *ctx, const sqrn_paramset *ps, const sqrn
                               double *out_fin, double *out_raw, uint8_t *out_flags, int8_t *dbn_code, int min_ccap)
 {
     return guarded(ctx, [&] { return sqrn_debug_run_impl(ctx, ps, in, mode, n_items, item_seq, init_off, init_stems, item_subopt, out_cap, out_stems, out_n, out_fin, out_raw, out_flags, dbn_code, min_ccap); });
+}
+
+// ------------------------------------------------------------- Nussinov
+// The DP and the backtrack of sqrn_nussinov.cuh.  Persistent CTAs, each with its own workspace slot, take the
+// sequences of a tier longest first from a counter.  Shared-memory tier: the whole triangle in shared memory, for
+// sequences up to nu_smem_max_n(opt-in limit) positions; global tier: the triangle in the CTA's slot in HBM.  K (int16)
+// is in the slot for both.  The whole workspace (the global tier's slots and the shared-memory tier's K) takes at most
+// NU_WORKSPACE_CAP bytes, but at least one global slot (1.28 GB at 16 000 nt; 11 MB at 1 500 nt).  The context keeps
+// it between calls at the exact size the largest call needed (re-allocating 4 GiB per call cost more than the 500 x
+// 300-1500 nt DP itself) and frees it in sqrn_ctx_destroy.  The two tiers run concurrently on two streams, so the short
+// sequences do not wait for the longest long one.
+constexpr int64_t NU_WORKSPACE_CAP = (int64_t)4 << 30;
+
+template <int TW, bool SMEM>
+__global__ void __launch_bounds__(TW * 32, 1)
+k_nussinov(NuBatch nb, NuLayout L)
+{
+    extern __shared__ __align__(16) unsigned char smem[];
+    int *s_item = (int *)(smem + L.item_off);
+    const int64_t slot = blockIdx.x;
+    double *tri = SMEM ? (double *)smem : nb.wd + slot * nb.slot_d;
+    double *prevbuf = SMEM ? nullptr : (double *)(smem + L.prev_off);
+    int16_t *K = nb.wk + slot * nb.slot_k;
+    double *sb = SMEM ? nullptr : nb.wbest + slot * nb.slot_s;
+    int16_t *sk = SMEM ? nullptr : nb.wbk + slot * nb.slot_s;
+    for (;;) {
+        if (threadIdx.x == 0) *s_item = atomicAdd(nb.counter, 1);
+        __syncthreads();
+        const int item = *s_item;
+        __syncthreads();
+        if (item >= nb.n_items) break;
+        nu_item<TW>(nb, nb.order[item], tri, prevbuf, L, smem, K, sb, sk);
+    }
+}
+
+static int64_t nu_round8(int64_t x) { return (x + 7) & ~(int64_t)7; }
+
+static int sqrn_nussinov_batch_impl(sqrn_ctx *ctx, int64_t n_seqs, const int64_t *offsets, const uint8_t *symbols,
+                                    const int64_t *stem_offsets, const int32_t *stems, const double *scores,
+                                    int32_t minloop, int64_t *pair_offsets, int32_t *pairs)
+{
+    if (!ctx) return SQRN_E_BADARG;
+    if (n_seqs < 0 || n_seqs >= (1LL << 31) || !offsets || !stem_offsets || !pair_offsets || minloop < 0 || offsets[0] != 0) {
+        ctx->err = "nussinov: bad arguments (offsets / stem_offsets / pair_offsets must be given, offsets[0] == 0, minloop >= 0)";
+        return SQRN_E_BADARG;
+    }
+    cudaSetDevice(ctx->device);
+    ctx->n_launches = 0; ctx->n_calls = 0; ctx->kernel_ms = 0; ctx->n_cluster_launches = 0;
+    std::vector<int64_t> out_base((size_t)n_seqs + 1, 0);
+    for (int64_t b = 0; b < n_seqs; b++) {
+        const int64_t n = offsets[b + 1] - offsets[b], ns = stem_offsets[b + 1] - stem_offsets[b];
+        if (n < 0 || n > SQRN_MAX_LEN || ns < 0) {
+            ctx->err = "nussinov: offsets must not decrease and a sequence may have at most SQRN_MAX_LEN positions";
+            return SQRN_E_BADARG;
+        }
+        if (ns > 0 && (!stems || !scores)) { ctx->err = "nussinov: stems / scores missing"; return SQRN_E_BADARG; }
+        if (ns > 0 && !nu_stems_ok((int)n, stems + 3 * stem_offsets[b], ns)) {
+            ctx->err = "nussinov: a stem of sequence " + std::to_string(b) + " leaves [0, N) or has len < 1";
+            return SQRN_E_BADARG;
+        }
+        out_base[(size_t)b + 1] = out_base[(size_t)b] + n / 2;
+    }
+    const int64_t total = offsets[n_seqs], cap = out_base[(size_t)n_seqs];
+    if ((total > 0 && !symbols) || (cap > 0 && !pairs)) { ctx->err = "nussinov: symbols / pairs missing"; return SQRN_E_BADARG; }
+    pair_offsets[0] = 0;
+    if (n_seqs == 0) return SQRN_OK;
+
+    // candidate lists P(j) per sequence (host threads), then one flat CSR: sequence b's column pointers at offsets[b] + b
+    std::vector<std::vector<int64_t>> cnt((size_t)n_seqs);
+    std::vector<std::vector<int16_t>> lk((size_t)n_seqs);
+    std::vector<std::vector<double>> le((size_t)n_seqs);
+    parallel_for(n_seqs, [&](int64_t b) {
+        nu_seq_lists((int)(offsets[b + 1] - offsets[b]), stems ? stems + 3 * stem_offsets[b] : nullptr,
+                     scores ? scores + stem_offsets[b] : nullptr, stem_offsets[b + 1] - stem_offsets[b], cnt[(size_t)b], lk[(size_t)b], le[(size_t)b]);
+    });
+    std::vector<int64_t> pbase((size_t)n_seqs + 1, 0);
+    for (int64_t b = 0; b < n_seqs; b++) pbase[(size_t)b + 1] = pbase[(size_t)b] + (int64_t)lk[(size_t)b].size();
+    std::vector<int64_t> colptr((size_t)(total + n_seqs));
+    std::vector<int16_t> pk((size_t)std::max<int64_t>(pbase[(size_t)n_seqs], 1));
+    std::vector<double> pe(pk.size());
+    parallel_for(n_seqs, [&](int64_t b) {
+        int64_t *cp = colptr.data() + offsets[b] + b, at = pbase[(size_t)b];
+        const int N = (int)(offsets[b + 1] - offsets[b]);
+        for (int j = 0; j < N; j++) { cp[j] = at; at += cnt[(size_t)b][(size_t)j]; }
+        cp[N] = at;
+        std::copy(lk[(size_t)b].begin(), lk[(size_t)b].end(), pk.begin() + pbase[(size_t)b]);
+        std::copy(le[(size_t)b].begin(), le[(size_t)b].end(), pe.begin() + pbase[(size_t)b]);
+    });
+
+    // the two tiers, each longest first; sequences of < 2 positions have no pair and are not launched
+    const int smax = nu_smem_max_n(ctx->smem_optin);
+    std::vector<int32_t> ord_g, ord_s;
+    for (int64_t b = 0; b < n_seqs; b++) {
+        const int64_t n = offsets[b + 1] - offsets[b];
+        if (n >= 2) (n <= smax ? ord_s : ord_g).push_back((int32_t)b);
+    }
+    auto longest_first = [&](int32_t a, int32_t c) { return offsets[a + 1] - offsets[a] > offsets[c + 1] - offsets[c]; };
+    std::stable_sort(ord_g.begin(), ord_g.end(), longest_first);
+    std::stable_sort(ord_s.begin(), ord_s.end(), longest_first);
+    std::vector<int32_t> order(ord_g);
+    order.insert(order.end(), ord_s.begin(), ord_s.end());
+
+    cudaStream_t st = ctx->stream;
+    NuBatch nb{};
+    int64_t *d_off, *d_colptr, *d_obase; uint8_t *d_sym; int16_t *d_pk; double *d_pe; int32_t *d_order, *d_outp, *d_outn; int *d_cnt;
+    TRY(upload(ctx, B_OFF, offsets, (size_t)n_seqs + 1, &d_off));
+    TRY(upload(ctx, B_SYM, symbols, (size_t)total, &d_sym));
+    TRY(upload(ctx, NU_COLPTR, colptr.data(), colptr.size(), &d_colptr));
+    TRY(upload(ctx, NU_PK, pk.data(), (size_t)pbase[(size_t)n_seqs], &d_pk));
+    TRY(upload(ctx, NU_PE, pe.data(), (size_t)pbase[(size_t)n_seqs], &d_pe));
+    TRY(upload(ctx, NU_ORDER, order.data(), order.size(), &d_order));
+    TRY(upload(ctx, NU_OUTBASE, out_base.data(), (size_t)n_seqs, &d_obase));
+    TRY(dalloc(ctx, NU_OUTP, (size_t)(2 * cap), &d_outp));
+    TRY(dalloc(ctx, NU_OUTN, (size_t)n_seqs, &d_outn));
+    TRY(dalloc(ctx, NU_CNT, 2, &d_cnt));
+    CK(cudaMemsetAsync(d_outn, 0, (size_t)n_seqs * sizeof(int32_t), st));
+    CK(cudaMemsetAsync(d_cnt, 0, 2 * sizeof(int), st));
+    nb.off = d_off; nb.sym = d_sym; nb.colptr = d_colptr; nb.pk = d_pk; nb.pe = d_pe; nb.minloop = minloop;
+    nb.out_base = d_obase; nb.out_pairs = d_outp; nb.out_n = d_outn;
+
+    // launch geometry first: one workspace for both tiers
+    const int ng = (int)ord_g.size(), nsm = (int)ord_s.size();
+    NuLayout Lg{}, Ls{};
+    int grid_g = 0, grid_s = 0;
+    int64_t kg = 0, ks = 0, slot_d = 0, slot_s = 0;
+    auto kern_g = k_nussinov<NU_GLOB_TW, false>;
+    auto kern_s = k_nussinov<NU_SMEM_TW, true>;
+    if (ng) {
+        const int nmax = (int)(offsets[ord_g[0] + 1] - offsets[ord_g[0]]);
+        Lg = nu_layout(nmax, false);
+        CK(cudaFuncSetAttribute(kern_g, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Lg.total));
+        int occ = 0;
+        CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern_g, NU_GLOB_TW * 32, Lg.total));
+        slot_d = nu_round8(nu_cells(nmax)); kg = nu_round8(nu_cells(nmax)); slot_s = nu_round8(nmax);
+        grid_g = (int)std::min<int64_t>((int64_t)ng, (int64_t)ctx->sm_count * std::max(occ, 1));
+    }
+    if (nsm) {
+        const int nmax = (int)(offsets[ord_s[0] + 1] - offsets[ord_s[0]]);
+        Ls = nu_layout(nmax, true);
+        CK(cudaFuncSetAttribute(kern_s, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Ls.total));
+        int occ = 0;
+        CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern_s, NU_SMEM_TW * 32, Ls.total));
+        ks = nu_round8(nu_cells(nmax));
+        grid_s = (int)std::min<int64_t>((int64_t)nsm, (int64_t)ctx->sm_count * std::max(occ, 1));
+    }
+    if (ng) {                                         // the global slots get what the shared tier's K leaves of the cap
+        const int64_t slot_bytes = 8 * slot_d + 2 * kg + 10 * slot_s;
+        grid_g = (int)std::min<int64_t>(grid_g, std::max<int64_t>(1, (NU_WORKSPACE_CAP - 2 * grid_s * ks) / slot_bytes));
+    }
+    // workspace: global-tier triangles | row best values | K of both tiers | row best k (each part 8-element aligned)
+    const int64_t n_wd = grid_g * slot_d, n_wb = grid_g * slot_s, n_wk = grid_g * kg + grid_s * ks, n_wbk = grid_g * slot_s;
+    const size_t ws_bytes = (size_t)(8 * (n_wd + n_wb) + 2 * (n_wk + n_wbk) + 16);
+    if (ws_bytes > ctx->nu_ws_bytes) {
+        if (ctx->nu_ws) cudaFree(ctx->nu_ws);
+        ctx->nu_ws = nullptr; ctx->nu_ws_bytes = 0;
+        CK(cudaMalloc(&ctx->nu_ws, ws_bytes));
+        ctx->nu_ws_bytes = ws_bytes;
+    }
+    double *d_wd = (double *)ctx->nu_ws, *d_wb = d_wd + n_wd;
+    int16_t *d_wk = (int16_t *)(d_wb + n_wb), *d_wbk = d_wk + n_wk;
+    CK(cudaEventRecord(ctx->ev0, st));
+    CK(cudaEventRecord(ctx->ev_start, st));          // the uploads are done: where the second stream starts
+    if (ng) {
+        NuBatch g = nb;
+        g.n_items = ng; g.order = d_order; g.counter = d_cnt;
+        g.wd = d_wd; g.wk = d_wk; g.wbest = d_wb; g.wbk = d_wbk; g.slot_d = slot_d; g.slot_k = kg; g.slot_s = slot_s;
+        kern_g<<<grid_g, NU_GLOB_TW * 32, Lg.total, st>>>(g, Lg);
+        CK(cudaGetLastError());
+        ctx->n_launches++;
+    }
+    if (nsm) {
+        // on the second stream, behind the uploads of the first: the two tiers share the SMs
+        NuBatch s = nb;
+        s.n_items = nsm; s.order = d_order + ng; s.counter = d_cnt + 1;
+        s.wk = d_wk + grid_g * kg; s.slot_k = ks;
+        CK(cudaStreamWaitEvent(ctx->s_k2, ctx->ev_start, 0));
+        kern_s<<<grid_s, NU_SMEM_TW * 32, Ls.total, ctx->s_k2>>>(s, Ls);
+        CK(cudaGetLastError());
+        CK(cudaEventRecord(ctx->ev_k2done, ctx->s_k2));
+        CK(cudaStreamWaitEvent(st, ctx->ev_k2done, 0));
+        ctx->n_launches++;
+    }
+    CK(cudaEventRecord(ctx->ev1, st));
+    std::vector<int32_t> outn((size_t)n_seqs);
+    CK(cudaMemcpyAsync(outn.data(), d_outn, (size_t)n_seqs * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+    if (cap > 0) CK(cudaMemcpyAsync(pairs, d_outp, (size_t)(2 * cap) * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+    CK(cudaStreamSynchronize(st));
+    float ms = 0.f;
+    if (cudaEventElapsedTime(&ms, ctx->ev0, ctx->ev1) == cudaSuccess) ctx->kernel_ms = ms;
+    // sequence b's pairs were written at out_base[b]; pack them in sequence order (in place: never moves right)
+    int64_t at = 0;
+    for (int64_t b = 0; b < n_seqs; b++) {
+        pair_offsets[b] = at;
+        const int64_t m = outn[(size_t)b];
+        if (m && at != out_base[(size_t)b]) memmove(pairs + 2 * at, pairs + 2 * out_base[(size_t)b], (size_t)m * 2 * sizeof(int32_t));
+        at += m;
+    }
+    pair_offsets[n_seqs] = at;
+    if (cap > at) memset(pairs + 2 * at, 0, (size_t)(cap - at) * 2 * sizeof(int32_t));     // (no stale device memory)
+    return SQRN_OK;
+}
+
+extern "C" int sqrn_nussinov_batch(sqrn_ctx *ctx, int64_t n_seqs, const int64_t *offsets, const uint8_t *symbols,
+                                   const int64_t *stem_offsets, const int32_t *stems, const double *scores,
+                                   int32_t minloop, int64_t *pair_offsets, int32_t *pairs)
+{
+    return guarded(ctx, [&] { return sqrn_nussinov_batch_impl(ctx, n_seqs, offsets, symbols, stem_offsets, stems, scores, minloop, pair_offsets, pairs); });
 }
