@@ -205,6 +205,25 @@ SQRN_API int  sqrn_nussinov_batch(sqrn_ctx *ctx, int64_t n_seqs, const int64_t *
                                   const int64_t *stem_offsets, const int32_t *stems, const double *scores,
                                   int32_t minloop, int64_t *pair_offsets, int32_t *pairs);
 
+/* The Hungarian builder (SQRNalgos.py: Hungarian, what RunAlgo runs for algorithm "H") for a batch, on the device: per
+ * sequence SciPy's linear_sum_assignment (rectangular_lsap.cpp) on the symmetric N x N matrix with cost -(score **
+ * power) at the pairs of its stems and 0 elsewhere, reproduced operation for operation (the same assignment, ties
+ * included), then the pairs (k, l) kept by the host builder: mutual, on a non-zero cell, and k < l - minloop or a
+ * separator ';' '&' of `symbols` between them.  No N x N matrix is formed.  Host buffers in and out.
+ *   offsets, symbols, stem_offsets, stems, scores, pair_offsets, pairs: as sqrn_nussinov_batch (pairs sorted by v);
+ *                a stem's pairs (i+t, j-t) must have i+t < j-t; a pair two stems hold takes the later stem's score;
+ *   minloop      >= 0 (RunAlgo passes 3);  power: the exponent of the weights (RunAlgo passes 1.7).
+ * SQRN_E_BADARG: a stem outside [0, N), with len < 1 or with a pair (v, w), v >= w; a sequence longer than
+ * SQRN_MAX_LEN; minloop < 0; a negative or NaN score; a non-finite score ** power (C pow; the host builder has complex
+ * numbers or an infeasible matrix there); a reduced cost that overflows (SciPy: infeasible).
+ * Sequences of up to 256 positions run a warp each, longer ones a CTA each with the state (42 bytes a position) in
+ * shared memory up to ~5 500 positions on a B200 (the opt-in limit), in a device workspace beyond (one slot per SM at
+ * most, 1.4 MB at SQRN_MAX_LEN, kept by the context until sqrn_ctx_destroy).  Longest first within each tier; the warp
+ * tier runs concurrently with the others.                                                                            */
+SQRN_API int  sqrn_hungarian_batch(sqrn_ctx *ctx, int64_t n_seqs, const int64_t *offsets, const uint8_t *symbols,
+                                   const int64_t *stem_offsets, const int32_t *stems, const double *scores,
+                                   int32_t minloop, double power, int64_t *pair_offsets, int32_t *pairs);
+
 /* ---- single-path fast lane (poollim == 1: `byseq pl=1`, SQUARNA.py:887-935) --
  * One parameter set, default reactivities, no restraints: one structure per
  * sequence, written as ASCII dot-bracket.  `symbols`/`offsets`/outputs are HOST

@@ -22,7 +22,8 @@ import re
 import numpy as np
 
 from . import _lib
-from ._lib import PackedBatch
+from ._abi import E_BADARG
+from ._lib import PackedBatch, SqrnError
 
 GAPS = {'-', '.', '~'}          # seq.py:12
 SEPS = {';', '&'}               # seq.py:14
@@ -624,7 +625,7 @@ def _cell_scorer(p, paramset, smat, bpp_mode=0, bpp_term=None):
 def RunAlgo(seq, stems, cell_score, minlen, minscore, algo="E", levellimit=3, pairs=None):
     """one non-greedy prediction (seq.py:548-595).  stems: AnnotateStems output [[pairs, len, score], ...];
     cell_score(v, w) = bpscorematrix[v, w].  pairs: what the builder returned when it ran elsewhere (the device
-    Nussinov builder); `stems` is then not read."""
+    Nussinov or Hungarian builder); `stems` is then not read."""
     from . import SQRNalgos
     N = len(seq)
     if pairs is not None:
@@ -682,18 +683,27 @@ def _predict_many_mixed(entries, paramsets, conslim, toplim, hardrest, rankbydif
             if others:
                 batch = _make_batch(preps, idx, comp, stemmatrix, interchainonly, bpp=bpp)
                 found = ctx.yield_stems(ps, batch)
-                # Nussinov on the device when the context has the builder (the host SQRNalgos.Nussinov otherwise): one
-                # call for the group, over the stems just enumerated; the stem lists are built only for E / H
+                # Nussinov and Hungarian on the device when the context has the builder (the host SQRNalgos functions
+                # otherwise): one call each for the group, over the stems just enumerated; the stem lists are built
+                # only for E and for a builder that runs on the host
                 nuss = getattr(ctx, "nussinov", None) if "N" in others else None
-                dev_pairs = nuss(batch.symbols, batch.offsets, found, minloop=3) if nuss is not None else None
-                lists = dev_pairs is None or any(a != "N" for a in others)
+                dev_pairs = {"N": nuss(batch.symbols, batch.offsets, found, minloop=3)} if nuss is not None else {}
+                hung = getattr(ctx, "hungarian", None) if "H" in others else None
+                if hung is not None:
+                    try:
+                        dev_pairs["H"] = hung(batch.symbols, batch.offsets, found, minloop=3, power=1.7)
+                    except SqrnError as e:
+                        # negative / NaN scores or non-finite weights: the host builder gives what it gives today
+                        if e.code != E_BADARG:
+                            raise
+                lists = any(a not in dev_pairs for a in others)
                 for q, (k, (st, sc)) in enumerate(zip(idx, found)):
                     p = preps[k]
                     stems = [[[(i + t, j - t) for t in range(ln)], ln, float(s_)] for (i, j, ln), s_ in zip(st.tolist(), sc.tolist())] if lists else None
                     cell = _cell_scorer(p, ps, smat_np, bpp[0] if bpp else 0, bpp[1][q] if bpp else None)
                     ll = levellimit if levellimit is not None else 3 - int(len(p.shortseq) > 500)
                     for algo in others:
-                        pairs = dev_pairs[q].tolist() if algo == "N" and dev_pairs is not None else None
+                        pairs = dev_pairs[algo][q].tolist() if algo in dev_pairs else None
                         stemset = RunAlgo(p.shortseq, stems, cell, ps["minlen"], ps["minbpscore"], algo, ll, pairs=pairs)
                         per_ps[k][psi].append((stemset, ScoreStruct(p.shortseq, stemset, p.shortreacts)))
             if "G" in use:
@@ -770,7 +780,7 @@ def predict_many(entries, paramsets, conslim=1, toplim=5, hardrest=False, rankby
     for psi, ps in enumerate(paramsets):
         use = set(algos) if algos else set(ps["algorithms"])
         if use - {"G"} or ps.get("bpp", 0):
-            # Nussinov / Hungarian / Edmonds sets: stems from the GPU, the builders on the host (SURVEY 8f-2);
+            # Nussinov / Hungarian / Edmonds sets: stems from the GPU, N and H on the device, E on the host (SURVEY 8f-2);
             # bpp sets: the probabilities come from the host (ViennaRNA or set_rna_module) as one term per
             # parameter set (SURVEY 8f-4), so the sets run one call each
             mixed = True
@@ -911,7 +921,7 @@ def SQRNdbnseq(seq, reacts=None, restraints=None, dbn=None,
 
     threads / mp only choose a multiprocessing layout in the reference and never
     change results; here the work is one batched GPU call.  Parameter sets that name Nussinov / Hungarian /
-    Edmonds get their stems from the GPU and run those builders on the host (SQRNalgos.py); `entropy=True`
+    Edmonds get their stems from the GPU; Nussinov and Hungarian run there too, Edmonds on the host (SQRNalgos.py); `entropy=True`
     returns the stem-matrix entropy string of the first parameter set."""
     if entropy:
         return Entropy(seq, reacts, restraints, paramsets[0], interchainonly, stemmatrix, M=M, B=B)

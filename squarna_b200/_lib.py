@@ -23,13 +23,17 @@ EXPORTS = ["sqrn_abi_version", "sqrn_device_count", "sqrn_ctx_create", "sqrn_ctx
            "sqrn_ctx_set_tuning", "sqrn_text_parse", "sqrn_text_ungap", "sqrn_text_format",
            "sqrn_fast_predict_packed_host", "sqrn_pack_symbols", "sqrn_unpack_dbn", "sqrn_fast_last_flags",
            "sqrn_stem_matrix_batch", "sqrn_fast_predict_packed_device", "sqrn_codes_to_ascii", "sqrn_dbn_pairs",
-           "sqrn_nussinov_batch"]
+           "sqrn_nussinov_batch", "sqrn_hungarian_batch"]
 
 _lib = None
 
 
 class SqrnError(RuntimeError):
-    pass
+    """a library call failed; `code` is its SQRN_E_* return code"""
+
+    def __init__(self, msg, code=None):
+        super().__init__(msg)
+        self.code = code
 
 
 def load():
@@ -64,6 +68,7 @@ def load():
     L.sqrn_fast_last_flags.argtypes = [vp, i64, vp]
     L.sqrn_stem_matrix_batch.argtypes = [vp, C.POINTER(ParamSet), C.POINTER(Batch), vp, C.c_double, i64, C.POINTER(i64), vp]
     L.sqrn_nussinov_batch.argtypes = [vp, i64, vp, vp, vp, vp, vp, i32, vp, vp]
+    L.sqrn_hungarian_batch.argtypes = [vp, i64, vp, vp, vp, vp, vp, i32, C.c_double, vp, vp]
     L.sqrn_ctx_last_stats.argtypes = [vp, C.POINTER(i64), C.POINTER(C.c_double), C.POINTER(i64)]
     L.sqrn_debug_run.argtypes = [vp, C.POINTER(ParamSet), C.POINTER(Batch), C.c_int, C.c_int] + [vp] * 11 + [C.c_int]
     L.sqrn_text_parse.argtypes = [vp, i64, C.c_int, C.POINTER(i64), C.POINTER(i64), i64, i64, vp, vp, vp, vp]
@@ -389,7 +394,7 @@ class Context:
 
     def _check(self, rc):
         if rc != OK:
-            raise SqrnError("libsqrn_b200 error %d: %s" % (rc, self.L.sqrn_last_error(self.h).decode()))
+            raise SqrnError("libsqrn_b200 error %d: %s" % (rc, self.L.sqrn_last_error(self.h).decode()), rc)
 
     def set_stream(self, cuda_stream):
         self._check(self.L.sqrn_ctx_set_stream(self.h, C.c_void_p(cuda_stream)))
@@ -530,11 +535,10 @@ class Context:
             break
         return [(st[off[b]:off[b + 1]].copy(), sc[off[b]:off[b + 1]].copy()) for b in range(n)]
 
-    def nussinov(self, symbols, offsets, stems, minloop=3):
-        """the Nussinov builder (SQRNalgos.Nussinov + BackTrack) on the device for a batch (include/sqrn.h:
-        sqrn_nussinov_batch).  symbols / offsets: the ungapped sequences as in PackedBatch; stems: per sequence
-        (stems (k,3) int32, scores (k,) float64), as yield_stems returns them.  Returns per sequence its base pairs as
-        an (n, 2) int32 array sorted by (v, w)."""
+    @staticmethod
+    def _builder_args(symbols, offsets, stems):
+        """(n, offsets, symbols, stem_offsets, stems, scores, pair_offsets, pairs) of a builder call: the inputs flat,
+        the outputs sized for N/2 pairs per sequence"""
         offsets = np.ascontiguousarray(offsets, np.int64)
         symbols = np.ascontiguousarray(symbols, np.uint8)
         n = len(offsets) - 1
@@ -544,6 +548,25 @@ class Context:
         sc = np.concatenate([np.asarray(x, np.float64).ravel() for _, x in stems] + [np.zeros(1)])
         po = np.zeros(n + 1, np.int64)
         pairs = np.zeros((max(int((np.diff(offsets) // 2).sum()), 1), 2), np.int32)
+        return n, offsets, symbols, so, st, sc, po, pairs
+
+    def hungarian(self, symbols, offsets, stems, minloop=3, power=1.7):
+        """the Hungarian builder (SQRNalgos.Hungarian: SciPy's linear_sum_assignment and the pair filter) on the
+        device for a batch (include/sqrn.h: sqrn_hungarian_batch).  Arguments as `nussinov`; power: the exponent of
+        the pair weights.  Returns per sequence its base pairs as an (n, 2) int32 array sorted by v.  Raises
+        SqrnError with code E_BADARG for input the host builder cannot take either (negative or NaN scores,
+        non-finite weights) as well as for malformed input."""
+        n, offsets, symbols, so, st, sc, po, pairs = self._builder_args(symbols, offsets, stems)
+        self._check(self.L.sqrn_hungarian_batch(self.h, n, ptr(offsets), ptr(symbols), ptr(so), ptr(st), ptr(sc),
+                                                int(minloop), float(power), ptr(po), ptr(pairs)))
+        return [pairs[po[b]:po[b + 1]] for b in range(n)]
+
+    def nussinov(self, symbols, offsets, stems, minloop=3):
+        """the Nussinov builder (SQRNalgos.Nussinov + BackTrack) on the device for a batch (include/sqrn.h:
+        sqrn_nussinov_batch).  symbols / offsets: the ungapped sequences as in PackedBatch; stems: per sequence
+        (stems (k,3) int32, scores (k,) float64), as yield_stems returns them.  Returns per sequence its base pairs as
+        an (n, 2) int32 array sorted by (v, w)."""
+        n, offsets, symbols, so, st, sc, po, pairs = self._builder_args(symbols, offsets, stems)
         self._check(self.L.sqrn_nussinov_batch(self.h, n, ptr(offsets), ptr(symbols), ptr(so), ptr(st), ptr(sc),
                                                int(minloop), ptr(po), ptr(pairs)))
         return [pairs[po[b]:po[b + 1]] for b in range(n)]

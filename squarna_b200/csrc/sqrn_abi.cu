@@ -19,6 +19,7 @@
 #include <vector>
 #include "sqrn_params.h"
 #include "sqrn_nussinov.cuh"
+#include "sqrn_hungarian.cuh"
 
 using namespace sqrn;
 
@@ -196,7 +197,8 @@ struct CachedStems {
 enum { B_OFF, B_OFF32, B_SYM, B_RCODE, B_RVALS, B_RFPOS, B_RFNEG, B_RCLASS, B_RBOFF, B_RB, B_SMAT, B_COLS, B_BPP, B_BPPOFF,
        W_ORDER, W_ISEQ, W_IOFF, W_ISTEMS, W_SUBOPT, W_COUNTER, W_OOFF, W_OSTEMS, W_ON, W_OFIN, W_ORAW,
        W_OFLAGS, W_DOFF, W_DBNA, W_DBNC, W_NCALLS, W_OVF, W_GENT, W_GBPS, W_GQB, W_GCNT, W_GCNT2, W_GSTAT, W_OVF2, W_RNDC, W_RNDL, W_BASE, W_BASEOFF, W_BASEN, W_BASEBEND, W_MAT, W_CELLCNT, W_CELLS, W_CELLS2,
-       NU_COLPTR, NU_PK, NU_PE, NU_ORDER, NU_OUTBASE, NU_OUTP, NU_OUTN, NU_CNT, NBUF };
+       NU_COLPTR, NU_PK, NU_PE, NU_ORDER, NU_OUTBASE, NU_OUTP, NU_OUTN, NU_CNT,
+       HU_ROWPTR, HU_ACOL, HU_ACOST, HU_ORDER, HU_OUTBASE, HU_OUTP, HU_OUTN, HU_CNT, NBUF };
 
 // ------------------------------------------------------------- launch plan
 struct Plan { int tw, threads, tpc, grid; size_t smem; Layout L; int fast_ncap = 0; int cluster = 0; bool cl_plain = false;
@@ -227,6 +229,7 @@ struct sqrn_ctx {
     int gl_rebuild = 0;          // tuning knob: rebuild period of the binned global list in passes (0: the default)
     CachedResult cres; CachedStems cstems;
     void *nu_ws = nullptr; size_t nu_ws_bytes = 0;   // workspace of sqrn_nussinov_batch (exact size, grown on demand)
+    void *hu_ws = nullptr; size_t hu_ws_bytes = 0;   // global-tier slots of sqrn_hungarian_batch (grown on demand)
 };
 
 static std::string g_create_err;
@@ -313,6 +316,7 @@ extern "C" void sqrn_ctx_destroy(sqrn_ctx *ctx)
     if (ctx->hflags) cudaFreeHost(ctx->hflags);
     if (ctx->horder) cudaFreeHost(ctx->horder);
     if (ctx->nu_ws) cudaFree(ctx->nu_ws);
+    if (ctx->hu_ws) cudaFree(ctx->hu_ws);
     delete ctx;
 }
 
@@ -2299,4 +2303,213 @@ extern "C" int sqrn_nussinov_batch(sqrn_ctx *ctx, int64_t n_seqs, const int64_t 
                                    int32_t minloop, int64_t *pair_offsets, int32_t *pairs)
 {
     return guarded(ctx, [&] { return sqrn_nussinov_batch_impl(ctx, n_seqs, offsets, symbols, stem_offsets, stems, scores, minloop, pair_offsets, pairs); });
+}
+
+// ------------------------------------------------------------- Hungarian
+// The assignment and the filter of sqrn_hungarian.cuh.  Three tiers by length, each a persistent kernel whose teams
+// take the tier's sequences longest first from a counter: a warp per sequence up to HU_WARP_MAX_N positions (HU_WPC
+// states in a CTA's shared memory), a CTA with its state in shared memory up to hu_smem_max_n(opt-in limit), and a CTA
+// with its state in a slot of a device workspace beyond that (at most one slot per SM: 1.4 MB at SQRN_MAX_LEN).  The
+// warp tier runs on the second stream, concurrently with the other two.
+template <int TW, bool SMEM>
+__global__ void __launch_bounds__(TW == 1 ? HU_WPC * 32 : TW * 32, 1)
+k_hungarian(HuBatch hb, HuLayout L)
+{
+    extern __shared__ __align__(16) unsigned char smem[];
+    if (TW == 1) {
+        unsigned char *st = smem + (threadIdx.x >> 5) * L.total;
+        for (;;) {
+            int item = 0;
+            if ((threadIdx.x & 31) == 0) item = atomicAdd(hb.counter, 1);
+            item = __shfl_sync(0xffffffffu, item, 0);
+            if (item >= hb.n_items) break;
+            hu_item<HuTeam<1>>(hb, hb.order[item], st, L, nullptr);
+        }
+        return;
+    }
+    const size_t base = SMEM ? L.total : 0;
+    HuKey *red = (HuKey *)(smem + base);
+    int *s_item = (int *)(smem + base + 16 * HU_CTA_TW);
+    unsigned char *st = SMEM ? smem : hb.ws + (int64_t)blockIdx.x * hb.slot_bytes;
+    for (;;) {
+        if (threadIdx.x == 0) *s_item = atomicAdd(hb.counter, 1);
+        __syncthreads();
+        const int item = *s_item;
+        __syncthreads();
+        if (item >= hb.n_items) break;
+        hu_item<HuTeam<TW>>(hb, hb.order[item], st, L, red);
+    }
+}
+
+static int sqrn_hungarian_batch_impl(sqrn_ctx *ctx, int64_t n_seqs, const int64_t *offsets, const uint8_t *symbols,
+                                     const int64_t *stem_offsets, const int32_t *stems, const double *scores,
+                                     int32_t minloop, double power, int64_t *pair_offsets, int32_t *pairs)
+{
+    if (!ctx) return SQRN_E_BADARG;
+    if (n_seqs < 0 || n_seqs >= (1LL << 31) || !offsets || !stem_offsets || !pair_offsets || minloop < 0 || offsets[0] != 0) {
+        ctx->err = "hungarian: bad arguments (offsets / stem_offsets / pair_offsets must be given, offsets[0] == 0, minloop >= 0)";
+        return SQRN_E_BADARG;
+    }
+    cudaSetDevice(ctx->device);
+    ctx->n_launches = 0; ctx->n_calls = 0; ctx->kernel_ms = 0; ctx->n_cluster_launches = 0;
+    std::vector<int64_t> out_base((size_t)n_seqs + 1, 0);
+    for (int64_t b = 0; b < n_seqs; b++) {
+        const int64_t n = offsets[b + 1] - offsets[b], ns = stem_offsets[b + 1] - stem_offsets[b];
+        if (n < 0 || n > SQRN_MAX_LEN || ns < 0) {
+            ctx->err = "hungarian: offsets must not decrease and a sequence may have at most SQRN_MAX_LEN positions";
+            return SQRN_E_BADARG;
+        }
+        if (ns > 0 && (!stems || !scores)) { ctx->err = "hungarian: stems / scores missing"; return SQRN_E_BADARG; }
+        if (ns > 0 && !hu_stems_ok((int)n, stems + 3 * stem_offsets[b], ns)) {
+            ctx->err = "hungarian: a stem of sequence " + std::to_string(b) + " leaves [0, N), has len < 1 or a pair (v, w) with v >= w";
+            return SQRN_E_BADARG;
+        }
+        out_base[(size_t)b + 1] = out_base[(size_t)b] + n / 2;
+    }
+    const int64_t total = offsets[n_seqs], cap = out_base[(size_t)n_seqs];
+    if ((total > 0 && !symbols) || (cap > 0 && !pairs)) { ctx->err = "hungarian: symbols / pairs missing"; return SQRN_E_BADARG; }
+    pair_offsets[0] = 0;
+    if (n_seqs == 0) return SQRN_OK;
+
+    // weights and adjacency per sequence (host threads), then one flat CSR: sequence b's row pointers at offsets[b] + b
+    std::vector<std::vector<int64_t>> rows((size_t)n_seqs);
+    std::vector<std::vector<int16_t>> acol((size_t)n_seqs);
+    std::vector<std::vector<double>> acost((size_t)n_seqs);
+    std::vector<char> bad((size_t)n_seqs, 0);
+    parallel_for(n_seqs, [&](int64_t b) {
+        const int64_t ns = stem_offsets[b + 1] - stem_offsets[b];
+        std::vector<double> w;
+        if (ns > 0 && !hu_weights(scores + stem_offsets[b], ns, power, w)) { bad[(size_t)b] = 1; return; }
+        hu_seq_adjacency((int)(offsets[b + 1] - offsets[b]), ns > 0 ? stems + 3 * stem_offsets[b] : nullptr, w.data(), ns,
+                         rows[(size_t)b], acol[(size_t)b], acost[(size_t)b]);
+    });
+    for (int64_t b = 0; b < n_seqs; b++)
+        if (bad[(size_t)b]) {
+            ctx->err = "hungarian: sequence " + std::to_string(b) + " has a negative or NaN score or a non-finite score ** power";
+            return SQRN_E_BADARG;
+        }
+    std::vector<int64_t> abase((size_t)n_seqs + 1, 0);
+    for (int64_t b = 0; b < n_seqs; b++) abase[(size_t)b + 1] = abase[(size_t)b] + (int64_t)acol[(size_t)b].size();
+    std::vector<int64_t> rowptr((size_t)(total + n_seqs));
+    std::vector<int16_t> ac((size_t)std::max<int64_t>(abase[(size_t)n_seqs], 1));
+    std::vector<double> ae(ac.size());
+    parallel_for(n_seqs, [&](int64_t b) {
+        int64_t *rp = rowptr.data() + offsets[b] + b;
+        const int N = (int)(offsets[b + 1] - offsets[b]);
+        for (int p = 0; p <= N; p++) rp[p] = abase[(size_t)b] + rows[(size_t)b][(size_t)p];
+        std::copy(acol[(size_t)b].begin(), acol[(size_t)b].end(), ac.begin() + abase[(size_t)b]);
+        std::copy(acost[(size_t)b].begin(), acost[(size_t)b].end(), ae.begin() + abase[(size_t)b]);
+    });
+
+    // the three tiers, each longest first; a sequence without stem pairs has no pair to keep and is not launched
+    const int smax = hu_smem_max_n(ctx->smem_optin);
+    std::vector<int32_t> ord[3];                      // global, CTA, warp
+    for (int64_t b = 0; b < n_seqs; b++) {
+        const int64_t n = offsets[b + 1] - offsets[b];
+        if (abase[(size_t)b + 1] > abase[(size_t)b]) ord[n > smax ? 0 : n > HU_WARP_MAX_N ? 1 : 2].push_back((int32_t)b);
+    }
+    auto longest_first = [&](int32_t a, int32_t c) { return offsets[a + 1] - offsets[a] > offsets[c + 1] - offsets[c]; };
+    std::vector<int32_t> order;
+    for (auto &o : ord) { std::stable_sort(o.begin(), o.end(), longest_first); order.insert(order.end(), o.begin(), o.end()); }
+
+    cudaStream_t st = ctx->stream;
+    int64_t *d_off, *d_rowptr, *d_obase; uint8_t *d_sym; int16_t *d_ac; double *d_ae; int32_t *d_order, *d_outp, *d_outn; int *d_cnt;
+    TRY(upload(ctx, B_OFF, offsets, (size_t)n_seqs + 1, &d_off));
+    TRY(upload(ctx, B_SYM, symbols, (size_t)total, &d_sym));
+    TRY(upload(ctx, HU_ROWPTR, rowptr.data(), rowptr.size(), &d_rowptr));
+    TRY(upload(ctx, HU_ACOL, ac.data(), (size_t)abase[(size_t)n_seqs], &d_ac));
+    TRY(upload(ctx, HU_ACOST, ae.data(), (size_t)abase[(size_t)n_seqs], &d_ae));
+    TRY(upload(ctx, HU_ORDER, order.data(), order.size(), &d_order));
+    TRY(upload(ctx, HU_OUTBASE, out_base.data(), (size_t)n_seqs, &d_obase));
+    TRY(dalloc(ctx, HU_OUTP, (size_t)(2 * cap), &d_outp));
+    TRY(dalloc(ctx, HU_OUTN, (size_t)n_seqs, &d_outn));
+    TRY(dalloc(ctx, HU_CNT, 3, &d_cnt));
+    CK(cudaMemsetAsync(d_outn, 0, (size_t)n_seqs * sizeof(int32_t), st));
+    CK(cudaMemsetAsync(d_cnt, 0, 3 * sizeof(int), st));
+    HuBatch hb{};
+    hb.off = d_off; hb.sym = d_sym; hb.rowptr = d_rowptr; hb.acol = d_ac; hb.acost = d_ae; hb.minloop = minloop;
+    hb.out_base = d_obase; hb.out_pairs = d_outp; hb.out_n = d_outn;
+
+    const int ng = (int)ord[0].size(), nc = (int)ord[1].size(), nw = (int)ord[2].size();
+    auto nmax = [&](const std::vector<int32_t> &o) { return (int)(offsets[o[0] + 1] - offsets[o[0]]); };
+    CK(cudaEventRecord(ctx->ev0, st));
+    CK(cudaEventRecord(ctx->ev_start, st));          // the uploads are done: where the second stream starts
+    if (nw) {                                         // warp tier, on the second stream
+        auto kern = k_hungarian<1, true>;
+        const HuLayout L = hu_layout(nmax(ord[2]));
+        const size_t sm = hu_warp_smem(nmax(ord[2]));
+        CK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm));
+        int occ = 0;
+        CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, HU_WPC * 32, sm));
+        HuBatch w = hb;
+        w.n_items = nw; w.order = d_order + ng + nc; w.counter = d_cnt + 2;
+        const int grid = (int)std::min<int64_t>((nw + HU_WPC - 1) / HU_WPC, (int64_t)ctx->sm_count * std::max(occ, 1));
+        CK(cudaStreamWaitEvent(ctx->s_k2, ctx->ev_start, 0));
+        kern<<<grid, HU_WPC * 32, sm, ctx->s_k2>>>(w, L);
+        CK(cudaGetLastError());
+        CK(cudaEventRecord(ctx->ev_k2done, ctx->s_k2));
+        ctx->n_launches++;
+    }
+    if (ng) {                                         // global tier: one slot per CTA, at most one CTA per SM
+        auto kern = k_hungarian<HU_CTA_TW, false>;
+        const HuLayout L = hu_layout(nmax(ord[0]));
+        const size_t sm = hu_cta_smem(0, false);
+        const int grid = std::min(ng, ctx->sm_count);
+        const size_t ws_bytes = (size_t)grid * L.total;
+        if (ws_bytes > ctx->hu_ws_bytes) {
+            if (ctx->hu_ws) cudaFree(ctx->hu_ws);
+            ctx->hu_ws = nullptr; ctx->hu_ws_bytes = 0;
+            CK(cudaMalloc(&ctx->hu_ws, ws_bytes));
+            ctx->hu_ws_bytes = ws_bytes;
+        }
+        HuBatch g = hb;
+        g.n_items = ng; g.order = d_order; g.counter = d_cnt; g.ws = (unsigned char *)ctx->hu_ws; g.slot_bytes = (int64_t)L.total;
+        kern<<<grid, HU_CTA_TW * 32, sm, st>>>(g, L);
+        CK(cudaGetLastError());
+        ctx->n_launches++;
+    }
+    if (nc) {                                         // CTA tier
+        auto kern = k_hungarian<HU_CTA_TW, true>;
+        const HuLayout L = hu_layout(nmax(ord[1]));
+        const size_t sm = hu_cta_smem(nmax(ord[1]), true);
+        CK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm));
+        int occ = 0;
+        CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, HU_CTA_TW * 32, sm));
+        HuBatch c = hb;
+        c.n_items = nc; c.order = d_order + ng; c.counter = d_cnt + 1;
+        const int grid = (int)std::min<int64_t>((int64_t)nc, (int64_t)ctx->sm_count * std::max(occ, 1));
+        kern<<<grid, HU_CTA_TW * 32, sm, st>>>(c, L);
+        CK(cudaGetLastError());
+        ctx->n_launches++;
+    }
+    if (nw) CK(cudaStreamWaitEvent(st, ctx->ev_k2done, 0));
+    CK(cudaEventRecord(ctx->ev1, st));
+    std::vector<int32_t> outn((size_t)n_seqs);
+    CK(cudaMemcpyAsync(outn.data(), d_outn, (size_t)n_seqs * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+    if (cap > 0) CK(cudaMemcpyAsync(pairs, d_outp, (size_t)(2 * cap) * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+    CK(cudaStreamSynchronize(st));
+    float ms = 0.f;
+    if (cudaEventElapsedTime(&ms, ctx->ev0, ctx->ev1) == cudaSuccess) ctx->kernel_ms = ms;
+    // sequence b's pairs were written at out_base[b]; pack them in sequence order (in place: never moves right)
+    int64_t at = 0;
+    for (int64_t b = 0; b < n_seqs; b++) {
+        pair_offsets[b] = at;
+        const int64_t m = outn[(size_t)b];
+        if (m < 0) {
+            ctx->err = "hungarian: sequence " + std::to_string(b) + ": the cost matrix is infeasible (a reduced cost overflows)";
+            return SQRN_E_BADARG;
+        }
+        if (m && at != out_base[(size_t)b]) memmove(pairs + 2 * at, pairs + 2 * out_base[(size_t)b], (size_t)m * 2 * sizeof(int32_t));
+        at += m;
+    }
+    pair_offsets[n_seqs] = at;
+    if (cap > at) memset(pairs + 2 * at, 0, (size_t)(cap - at) * 2 * sizeof(int32_t));     // (no stale device memory)
+    return SQRN_OK;
+}
+
+extern "C" int sqrn_hungarian_batch(sqrn_ctx *ctx, int64_t n_seqs, const int64_t *offsets, const uint8_t *symbols,
+                                    const int64_t *stem_offsets, const int32_t *stems, const double *scores,
+                                    int32_t minloop, double power, int64_t *pair_offsets, int32_t *pairs)
+{
+    return guarded(ctx, [&] { return sqrn_hungarian_batch_impl(ctx, n_seqs, offsets, symbols, stem_offsets, stems, scores, minloop, power, pair_offsets, pairs); });
 }

@@ -88,6 +88,13 @@ struct NuBatch {
 // One sequence: the column sweep (whole team), then the backtrack (one thread).  tri: the triangle (shared memory or
 // the workspace slot); prevbuf: NULL when the previous column is read in place (shared-memory tier), else a shared
 // copy of it; smem: the layout's base (staged candidates, backtrack scratch); K: the slot's int16 triangle.
+// pre[p] = separators ';' '&' among the first p symbols, p = 0 .. N
+__host__ __device__ inline void sep_prefix(const uint8_t *sq, int N, int32_t *pre)
+{
+    pre[0] = 0;
+    for (int p = 0; p < N; p++) pre[p + 1] = pre[p] + (sq[p] == ';' || sq[p] == '&');
+}
+
 template <int TW>
 __device__ void nu_item(const NuBatch &nb, int seq, double *tri, double *prevbuf, const NuLayout &L, unsigned char *smem,
                         int16_t *K, double *sbest, int16_t *sbk)
@@ -154,8 +161,8 @@ __device__ void nu_item(const NuBatch &nb, int seq, double *tri, double *prevbuf
         int32_t *pre = (int32_t *)smem;
         int32_t *partner = (int32_t *)(smem + nu_al(4 * (size_t)(N + 1)));
         int32_t *stk = (int32_t *)(smem + nu_al(4 * (size_t)(N + 1)) + nu_al(4 * (size_t)N));
-        pre[0] = 0;
-        for (int p = 0; p < N; p++) { pre[p + 1] = pre[p] + (sq[p] == ';' || sq[p] == '&'); partner[p] = -1; }
+        sep_prefix(sq, N, pre);
+        for (int p = 0; p < N; p++) partner[p] = -1;
         const int ml = nb.minloop;
         // a separator in [lo, hi)
         auto sep = [&](int lo_, int hi_) { return hi_ > lo_ && pre[hi_] - pre[lo_] > 0; };
@@ -197,27 +204,39 @@ inline bool nu_stems_ok(int N, const int32_t *st, int64_t ns)
     return true;
 }
 
-// P(j) of one sequence: counts[j] partners per column, then k ascending within each column, energies -score.  A pair
-// that two stems hold takes the score of the later stem (what a dict filled in stem order keeps).  Pairs with
-// k >= j - 1 can never be taken and are left out.
+// The pairs (k, j), k + min_span <= j, of the stems of one sequence, each once with the index of the LAST stem that
+// holds it (what a dict filled in stem order keeps), sorted by (j, k).  A key is j (SP_J bits) | k | stem index: 15 bits
+// each for positions up to SQRN_MAX_LEN, 34 for the stem.
+constexpr int SP_J = 49, SP_K = 34;
+constexpr uint64_t SP_POS = 0x7fff, SP_STEM = (1ull << SP_K) - 1;
+
+inline void stem_pair_keys(const int32_t *st, int64_t ns, int min_span, std::vector<uint64_t> &out)
+{
+    std::vector<uint64_t> keys;
+    for (int64_t s = 0; s < ns; s++)
+        for (int t = 0; t < st[3 * s + 2]; t++) {
+            const int64_t k = st[3 * s] + t, j = st[3 * s + 1] - t;
+            if (k + min_span <= j) keys.push_back((uint64_t)j << SP_J | (uint64_t)k << SP_K | (uint64_t)s);
+        }
+    std::sort(keys.begin(), keys.end());
+    out.clear();
+    for (size_t q = 0; q < keys.size(); q++)
+        if (q + 1 == keys.size() || keys[q + 1] >> SP_K != keys[q] >> SP_K) out.push_back(keys[q]);   // else a later stem holds it too
+}
+
+// P(j) of one sequence: counts[j] partners per column, then k ascending within each column, energies -score.  Pairs
+// with k >= j - 1 can never be taken and are left out.
 inline void nu_seq_lists(int N, const int32_t *st, const double *sc, int64_t ns, std::vector<int64_t> &counts,
                          std::vector<int16_t> &pk, std::vector<double> &pe)
 {
-    std::vector<uint64_t> keys;         // j (14 bits) | k (14 bits) | stem index (36 bits)
-    for (int64_t s = 0; s < ns; s++)
-        for (int t = 0; t < st[3 * s + 2]; t++) {
-            const uint64_t k = (uint64_t)(st[3 * s] + t), j = (uint64_t)(st[3 * s + 1] - t);
-            if (k + 1 < j) keys.push_back(j << 50 | k << 36 | (uint64_t)s);
-        }
-    std::sort(keys.begin(), keys.end());
+    std::vector<uint64_t> keys;
+    stem_pair_keys(st, ns, 2, keys);
     counts.assign((size_t)N, 0);
     pk.clear(); pe.clear();
-    for (size_t q = 0; q < keys.size(); q++) {
-        if (q + 1 < keys.size() && keys[q + 1] >> 36 == keys[q] >> 36) continue;      // the later stem holds it too
-        const int j = (int)(keys[q] >> 50), k = (int)(keys[q] >> 36 & 0x3fff);
-        counts[(size_t)j]++;
-        pk.push_back((int16_t)k);
-        pe.push_back(-sc[keys[q] & 0xfffffffffull]);
+    for (const uint64_t key : keys) {
+        counts[(size_t)(key >> SP_J)]++;
+        pk.push_back((int16_t)(key >> SP_K & SP_POS));
+        pe.push_back(-sc[key & SP_STEM]);
     }
 }
 
