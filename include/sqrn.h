@@ -224,6 +224,24 @@ SQRN_API int  sqrn_hungarian_batch(sqrn_ctx *ctx, int64_t n_seqs, const int64_t 
                                    const int64_t *stem_offsets, const int32_t *stems, const double *scores,
                                    int32_t minloop, double power, int64_t *pair_offsets, int32_t *pairs);
 
+/* The Edmonds builder (SQRNalgos.py: Edmonds, what RunAlgo runs for algorithm "E") for a batch, on the device: per
+ * sequence NetworkX's max_weight_matching (networkx/algorithms/matching.py, maxcardinality False) on the graph whose
+ * edges are the pairs of its stems, weight score ** power, reproduced statement for statement (the same matching, ties
+ * included).  An edge sits at the first occurrence of its pair in stem order and takes the last stem's score; the nodes
+ * and each node's adjacency keep NetworkX's insertion order.  No pair filter.  Host buffers in and out.
+ *   offsets, stem_offsets, stems, scores, pair_offsets, pairs: as sqrn_hungarian_batch (no symbols); pairs (v, w),
+ *                v < w, sorted by v;  power: the exponent of the weights (RunAlgo passes 1.7).
+ * SQRN_E_BADARG: a stem outside [0, N), with len < 1 or with a pair (v, w), v >= w; a sequence longer than
+ * SQRN_MAX_LEN; a negative or NaN score; a score ** power (C pow) that is not finite or above DBL_MAX / 4 (the host
+ * builder has complex numbers or overflows there).
+ * Sequences of up to 256 positions run a warp each, longer ones a CTA each with the node state (~124 bytes a node) in
+ * shared memory up to 1 933 positions on a B200 (the opt-in limit), in a device workspace beyond.  Every team keeps
+ * 16 bytes an edge in the workspace (at most 4 GiB, kept by the context until sqrn_ctx_destroy).  Longest first
+ * within each tier; the warp tier runs concurrently with the others.                                                 */
+SQRN_API int  sqrn_edmonds_batch(sqrn_ctx *ctx, int64_t n_seqs, const int64_t *offsets, const int64_t *stem_offsets,
+                                 const int32_t *stems, const double *scores, double power, int64_t *pair_offsets,
+                                 int32_t *pairs);
+
 /* ---- single-path fast lane (poollim == 1: `byseq pl=1`, SQUARNA.py:887-935) --
  * One parameter set, default reactivities, no restraints: one structure per
  * sequence, written as ASCII dot-bracket.  `symbols`/`offsets`/outputs are HOST

@@ -1,9 +1,9 @@
 """The non-greedy structure builders of SQUARNA (Nussinov / Hungarian / Edmonds, SQRNalgos.py in the reference),
-fed by the stems the GPU enumerates (sqrn_yield_stems_batch = AnnotateStems).  SURVEY.md 8(f)-2: Edmonds is
-NetworkX on the host.  Nussinov and Hungarian run on the device when the caller has a library context
-(sqrn_nussinov_batch, csrc/sqrn_nussinov.cuh, DESIGN.md 3.8; sqrn_hungarian_batch, csrc/sqrn_hungarian.cuh, 3.9); the
-functions here are the specifications the device code reproduces pair for pair (tests/test_nussinov.py,
-tests/test_hungarian.py) and the path of contexts without the device builders.  Results are pinned to the reference by
+fed by the stems the GPU enumerates (sqrn_yield_stems_batch = AnnotateStems).  SURVEY.md 8(f)-2.  All three run on
+the device when the caller has a library context (sqrn_nussinov_batch, csrc/sqrn_nussinov.cuh, DESIGN.md 3.8;
+sqrn_hungarian_batch, csrc/sqrn_hungarian.cuh, 3.9; sqrn_edmonds_batch, csrc/sqrn_edmonds.cuh, 3.10); the functions
+here are the specifications the device code reproduces pair for pair (tests/test_nussinov.py, tests/test_hungarian.py,
+tests/test_edmonds.py) and the path of contexts without the device builders.  Results are pinned to the reference by
 tests/golden/algos.json (tests/golden/make_golden.py algos).
 
 Every function takes `stems` = [[pairs, length, score], ...] in AnnotateStems order and returns base pairs."""

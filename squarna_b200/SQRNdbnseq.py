@@ -625,7 +625,7 @@ def _cell_scorer(p, paramset, smat, bpp_mode=0, bpp_term=None):
 def RunAlgo(seq, stems, cell_score, minlen, minscore, algo="E", levellimit=3, pairs=None):
     """one non-greedy prediction (seq.py:548-595).  stems: AnnotateStems output [[pairs, len, score], ...];
     cell_score(v, w) = bpscorematrix[v, w].  pairs: what the builder returned when it ran elsewhere (the device
-    Nussinov or Hungarian builder); `stems` is then not read."""
+    Nussinov, Hungarian or Edmonds builder); `stems` is then not read."""
     from . import SQRNalgos
     N = len(seq)
     if pairs is not None:
@@ -683,17 +683,19 @@ def _predict_many_mixed(entries, paramsets, conslim, toplim, hardrest, rankbydif
             if others:
                 batch = _make_batch(preps, idx, comp, stemmatrix, interchainonly, bpp=bpp)
                 found = ctx.yield_stems(ps, batch)
-                # Nussinov and Hungarian on the device when the context has the builder (the host SQRNalgos functions
-                # otherwise): one call each for the group, over the stems just enumerated; the stem lists are built
-                # only for E and for a builder that runs on the host
+                # Nussinov, Hungarian and Edmonds on the device when the context has the builder (the host SQRNalgos
+                # functions otherwise): one call each for the group, over the stems just enumerated; the stem lists are
+                # built only for a builder that runs on the host
                 nuss = getattr(ctx, "nussinov", None) if "N" in others else None
                 dev_pairs = {"N": nuss(batch.symbols, batch.offsets, found, minloop=3)} if nuss is not None else {}
-                hung = getattr(ctx, "hungarian", None) if "H" in others else None
-                if hung is not None:
+                for algo, name, kw in (("H", "hungarian", dict(minloop=3, power=1.7)), ("E", "edmonds", dict(power=1.7))):
+                    build = getattr(ctx, name, None) if algo in others else None
+                    if build is None:
+                        continue
                     try:
-                        dev_pairs["H"] = hung(batch.symbols, batch.offsets, found, minloop=3, power=1.7)
+                        dev_pairs[algo] = build(batch.symbols, batch.offsets, found, **kw)
                     except SqrnError as e:
-                        # negative / NaN scores or non-finite weights: the host builder gives what it gives today
+                        # negative / NaN scores or non-finite / huge weights: the host builder gives what it gives today
                         if e.code != E_BADARG:
                             raise
                 lists = any(a not in dev_pairs for a in others)
@@ -780,7 +782,7 @@ def predict_many(entries, paramsets, conslim=1, toplim=5, hardrest=False, rankby
     for psi, ps in enumerate(paramsets):
         use = set(algos) if algos else set(ps["algorithms"])
         if use - {"G"} or ps.get("bpp", 0):
-            # Nussinov / Hungarian / Edmonds sets: stems from the GPU, N and H on the device, E on the host (SURVEY 8f-2);
+            # Nussinov / Hungarian / Edmonds sets: stems and the builders on the GPU (SURVEY 8f-2);
             # bpp sets: the probabilities come from the host (ViennaRNA or set_rna_module) as one term per
             # parameter set (SURVEY 8f-4), so the sets run one call each
             mixed = True
@@ -921,7 +923,7 @@ def SQRNdbnseq(seq, reacts=None, restraints=None, dbn=None,
 
     threads / mp only choose a multiprocessing layout in the reference and never
     change results; here the work is one batched GPU call.  Parameter sets that name Nussinov / Hungarian /
-    Edmonds get their stems from the GPU; Nussinov and Hungarian run there too, Edmonds on the host (SQRNalgos.py); `entropy=True`
+    Edmonds get their stems from the GPU, and those builders run there too (SQRNalgos.py is the reference); `entropy=True`
     returns the stem-matrix entropy string of the first parameter set."""
     if entropy:
         return Entropy(seq, reacts, restraints, paramsets[0], interchainonly, stemmatrix, M=M, B=B)

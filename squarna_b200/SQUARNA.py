@@ -11,8 +11,8 @@ Behavioural differences from the reference, all outside the hot path:
     prints in input order.
   * parameter sets with `bpp != 0` (ViennaRNA, not installed: parity unpinned) and the
     rfam/g4/rbp restraint discovery (external binaries / network) raise NotImplementedError.
-    Nussinov / Hungarian / Edmonds parameter sets build on GPU-enumerated stems: Nussinov and Hungarian on the
-    device, Edmonds on the host.
+    Nussinov / Hungarian / Edmonds parameter sets build on GPU-enumerated stems, and the three builders run on the
+    device too.
 """
 import os
 import sys

@@ -23,7 +23,7 @@ EXPORTS = ["sqrn_abi_version", "sqrn_device_count", "sqrn_ctx_create", "sqrn_ctx
            "sqrn_ctx_set_tuning", "sqrn_text_parse", "sqrn_text_ungap", "sqrn_text_format",
            "sqrn_fast_predict_packed_host", "sqrn_pack_symbols", "sqrn_unpack_dbn", "sqrn_fast_last_flags",
            "sqrn_stem_matrix_batch", "sqrn_fast_predict_packed_device", "sqrn_codes_to_ascii", "sqrn_dbn_pairs",
-           "sqrn_nussinov_batch", "sqrn_hungarian_batch"]
+           "sqrn_nussinov_batch", "sqrn_hungarian_batch", "sqrn_edmonds_batch"]
 
 _lib = None
 
@@ -69,6 +69,7 @@ def load():
     L.sqrn_stem_matrix_batch.argtypes = [vp, C.POINTER(ParamSet), C.POINTER(Batch), vp, C.c_double, i64, C.POINTER(i64), vp]
     L.sqrn_nussinov_batch.argtypes = [vp, i64, vp, vp, vp, vp, vp, i32, vp, vp]
     L.sqrn_hungarian_batch.argtypes = [vp, i64, vp, vp, vp, vp, vp, i32, C.c_double, vp, vp]
+    L.sqrn_edmonds_batch.argtypes = [vp, i64, vp, vp, vp, vp, C.c_double, vp, vp]
     L.sqrn_ctx_last_stats.argtypes = [vp, C.POINTER(i64), C.POINTER(C.c_double), C.POINTER(i64)]
     L.sqrn_debug_run.argtypes = [vp, C.POINTER(ParamSet), C.POINTER(Batch), C.c_int, C.c_int] + [vp] * 11 + [C.c_int]
     L.sqrn_text_parse.argtypes = [vp, i64, C.c_int, C.POINTER(i64), C.POINTER(i64), i64, i64, vp, vp, vp, vp]
@@ -559,6 +560,17 @@ class Context:
         n, offsets, symbols, so, st, sc, po, pairs = self._builder_args(symbols, offsets, stems)
         self._check(self.L.sqrn_hungarian_batch(self.h, n, ptr(offsets), ptr(symbols), ptr(so), ptr(st), ptr(sc),
                                                 int(minloop), float(power), ptr(po), ptr(pairs)))
+        return [pairs[po[b]:po[b + 1]] for b in range(n)]
+
+    def edmonds(self, symbols, offsets, stems, power=1.7):
+        """the Edmonds builder (SQRNalgos.Edmonds: NetworkX's max_weight_matching on the stem pairs) on the device for
+        a batch (include/sqrn.h: sqrn_edmonds_batch).  Arguments as `hungarian` (the symbols only give the shape of
+        the batch).  Returns per sequence the matched pairs as an (n, 2) int32 array of (v, w), v < w, sorted by v.
+        Raises SqrnError with code E_BADARG for input the host builder cannot take either (negative or NaN scores,
+        non-finite or huge weights) as well as for malformed input."""
+        n, offsets, symbols, so, st, sc, po, pairs = self._builder_args(symbols, offsets, stems)
+        self._check(self.L.sqrn_edmonds_batch(self.h, n, ptr(offsets), ptr(so), ptr(st), ptr(sc), float(power),
+                                              ptr(po), ptr(pairs)))
         return [pairs[po[b]:po[b + 1]] for b in range(n)]
 
     def nussinov(self, symbols, offsets, stems, minloop=3):

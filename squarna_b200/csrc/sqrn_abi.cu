@@ -20,6 +20,7 @@
 #include "sqrn_params.h"
 #include "sqrn_nussinov.cuh"
 #include "sqrn_hungarian.cuh"
+#include "sqrn_edmonds.cuh"
 
 using namespace sqrn;
 
@@ -198,7 +199,8 @@ enum { B_OFF, B_OFF32, B_SYM, B_RCODE, B_RVALS, B_RFPOS, B_RFNEG, B_RCLASS, B_RB
        W_ORDER, W_ISEQ, W_IOFF, W_ISTEMS, W_SUBOPT, W_COUNTER, W_OOFF, W_OSTEMS, W_ON, W_OFIN, W_ORAW,
        W_OFLAGS, W_DOFF, W_DBNA, W_DBNC, W_NCALLS, W_OVF, W_GENT, W_GBPS, W_GQB, W_GCNT, W_GCNT2, W_GSTAT, W_OVF2, W_RNDC, W_RNDL, W_BASE, W_BASEOFF, W_BASEN, W_BASEBEND, W_MAT, W_CELLCNT, W_CELLS, W_CELLS2,
        NU_COLPTR, NU_PK, NU_PE, NU_ORDER, NU_OUTBASE, NU_OUTP, NU_OUTN, NU_CNT,
-       HU_ROWPTR, HU_ACOL, HU_ACOST, HU_ORDER, HU_OUTBASE, HU_OUTP, HU_OUTN, HU_CNT, NBUF };
+       HU_ROWPTR, HU_ACOL, HU_ACOST, HU_ORDER, HU_OUTBASE, HU_OUTP, HU_OUTN, HU_CNT,
+       ED_VBASE, ED_EBASE, ED_ROWPTR, ED_POS, ED_ADJ, ED_EP, ED_WT, ED_MAXW, ED_ORDER, ED_OUTBASE, ED_OUTP, ED_OUTN, ED_CNT, NBUF };
 
 // ------------------------------------------------------------- launch plan
 struct Plan { int tw, threads, tpc, grid; size_t smem; Layout L; int fast_ncap = 0; int cluster = 0; bool cl_plain = false;
@@ -230,6 +232,7 @@ struct sqrn_ctx {
     CachedResult cres; CachedStems cstems;
     void *nu_ws = nullptr; size_t nu_ws_bytes = 0;   // workspace of sqrn_nussinov_batch (exact size, grown on demand)
     void *hu_ws = nullptr; size_t hu_ws_bytes = 0;   // global-tier slots of sqrn_hungarian_batch (grown on demand)
+    void *ed_ws = nullptr; size_t ed_ws_bytes = 0;   // team slots of sqrn_edmonds_batch (grown on demand)
 };
 
 static std::string g_create_err;
@@ -317,6 +320,7 @@ extern "C" void sqrn_ctx_destroy(sqrn_ctx *ctx)
     if (ctx->horder) cudaFreeHost(ctx->horder);
     if (ctx->nu_ws) cudaFree(ctx->nu_ws);
     if (ctx->hu_ws) cudaFree(ctx->hu_ws);
+    if (ctx->ed_ws) cudaFree(ctx->ed_ws);
     delete ctx;
 }
 
@@ -2512,4 +2516,266 @@ extern "C" int sqrn_hungarian_batch(sqrn_ctx *ctx, int64_t n_seqs, const int64_t
                                     int32_t minloop, double power, int64_t *pair_offsets, int32_t *pairs)
 {
     return guarded(ctx, [&] { return sqrn_hungarian_batch_impl(ctx, n_seqs, offsets, symbols, stem_offsets, stems, scores, minloop, power, pair_offsets, pairs); });
+}
+
+// ------------------------------------------------------------- Edmonds
+// The matching of sqrn_edmonds.cuh.  Three tiers by length, each a persistent kernel whose teams take the tier's
+// sequences longest first from a counter: a warp per sequence up to ED_WARP_MAX_N positions (ED_WPC node states in a
+// CTA's shared memory), a CTA with its node state in shared memory up to ed_smem_max_n(opt-in limit), and a CTA with its
+// node state in its workspace slot beyond that.  Every team also has the edge state of its sequences (allowed-edge
+// stamps, the mybestedges arena) in its slot.  Slots are sized from the V and E of the launch's sequences; the whole
+// workspace takes at most ED_WORKSPACE_CAP bytes but at least one slot per tier, and the context keeps it between calls.
+// The adjacency is read-only, in global memory.  The warp tier runs on the second stream, concurrently with the others.
+constexpr int64_t ED_WORKSPACE_CAP = (int64_t)4 << 30;
+
+template <int TW, bool SMEM>
+__global__ void __launch_bounds__(TW == 1 ? ED_WPC * 32 : TW * 32, 1)
+k_edmonds(EdBatch eb, int64_t vbytes)
+{
+    extern __shared__ __align__(16) unsigned char smem[];
+    if (TW == 1) {
+        const int w = threadIdx.x >> 5;
+        unsigned char *st = smem + w * vbytes;
+        int32_t *est = (int32_t *)(eb.ws + ((int64_t)blockIdx.x * ED_WPC + w) * eb.slot_bytes);
+        for (;;) {
+            int item = 0;
+            if ((threadIdx.x & 31) == 0) item = atomicAdd(eb.counter, 1);
+            item = __shfl_sync(0xffffffffu, item, 0);
+            if (item >= eb.n_items) break;
+            ed_item<HuTeam<1>>(eb, eb.order[item], st, est, nullptr);
+        }
+        return;
+    }
+    const size_t base = SMEM ? vbytes : 0;
+    HuKey *red = (HuKey *)(smem + base);
+    int *s_item = (int *)(smem + base + 16 * ED_CTA_TW);
+    unsigned char *slot = eb.ws + (int64_t)blockIdx.x * eb.slot_bytes;
+    unsigned char *st = SMEM ? smem : slot;
+    int32_t *est = (int32_t *)(SMEM ? slot : slot + vbytes);
+    for (;;) {
+        if (threadIdx.x == 0) *s_item = atomicAdd(eb.counter, 1);
+        __syncthreads();
+        const int item = *s_item;
+        __syncthreads();
+        if (item >= eb.n_items) break;
+        ed_item<HuTeam<TW>>(eb, eb.order[item], st, est, red);
+    }
+}
+
+static int sqrn_edmonds_batch_impl(sqrn_ctx *ctx, int64_t n_seqs, const int64_t *offsets, const int64_t *stem_offsets,
+                                   const int32_t *stems, const double *scores, double power, int64_t *pair_offsets,
+                                   int32_t *pairs)
+{
+    if (!ctx) return SQRN_E_BADARG;
+    if (n_seqs < 0 || n_seqs >= (1LL << 31) || !offsets || !stem_offsets || !pair_offsets || offsets[0] != 0) {
+        ctx->err = "edmonds: bad arguments (offsets / stem_offsets / pair_offsets must be given, offsets[0] == 0)";
+        return SQRN_E_BADARG;
+    }
+    cudaSetDevice(ctx->device);
+    ctx->n_launches = 0; ctx->n_calls = 0; ctx->kernel_ms = 0; ctx->n_cluster_launches = 0;
+    std::vector<int64_t> out_base((size_t)n_seqs + 1, 0);
+    for (int64_t b = 0; b < n_seqs; b++) {
+        const int64_t n = offsets[b + 1] - offsets[b], ns = stem_offsets[b + 1] - stem_offsets[b];
+        if (n < 0 || n > SQRN_MAX_LEN || ns < 0) {
+            ctx->err = "edmonds: offsets must not decrease and a sequence may have at most SQRN_MAX_LEN positions";
+            return SQRN_E_BADARG;
+        }
+        if (ns > 0 && (!stems || !scores)) { ctx->err = "edmonds: stems / scores missing"; return SQRN_E_BADARG; }
+        if (ns > 0 && !hu_stems_ok((int)n, stems + 3 * stem_offsets[b], ns)) {
+            ctx->err = "edmonds: a stem of sequence " + std::to_string(b) + " leaves [0, N), has len < 1 or a pair (v, w) with v >= w";
+            return SQRN_E_BADARG;
+        }
+        out_base[(size_t)b + 1] = out_base[(size_t)b] + n / 2;
+    }
+    const int64_t cap = out_base[(size_t)n_seqs];
+    if (cap > 0 && !pairs) { ctx->err = "edmonds: pairs missing"; return SQRN_E_BADARG; }
+    pair_offsets[0] = 0;
+    if (n_seqs == 0) return SQRN_OK;
+
+    // the graph of each sequence (host threads), then flat arrays: nodes at vbase[b], edges at ebase[b], row pointers
+    // at vbase[b] + b holding offsets into the flat adjacency
+    std::vector<std::vector<int32_t>> pos((size_t)n_seqs), adj((size_t)n_seqs), ep((size_t)n_seqs);
+    std::vector<std::vector<int64_t>> rows((size_t)n_seqs);
+    std::vector<std::vector<double>> wt((size_t)n_seqs);
+    std::vector<double> maxw((size_t)n_seqs, 0.0);
+    std::vector<char> bad((size_t)n_seqs, 0);
+    parallel_for(n_seqs, [&](int64_t b) {
+        const int64_t ns = stem_offsets[b + 1] - stem_offsets[b];
+        std::vector<double> w;
+        if (ns > 0 && !ed_weights(scores + stem_offsets[b], ns, power, w)) { bad[(size_t)b] = 1; return; }
+        maxw[(size_t)b] = ed_seq_graph((int)(offsets[b + 1] - offsets[b]), ns > 0 ? stems + 3 * stem_offsets[b] : nullptr,
+                                       w.data(), ns, pos[(size_t)b], rows[(size_t)b], adj[(size_t)b], ep[(size_t)b], wt[(size_t)b]);
+    });
+    for (int64_t b = 0; b < n_seqs; b++)
+        if (bad[(size_t)b]) {
+            ctx->err = "edmonds: sequence " + std::to_string(b) + " has a negative or NaN score or a non-finite or huge score ** power";
+            return SQRN_E_BADARG;
+        }
+    std::vector<int64_t> vbase((size_t)n_seqs + 1, 0), ebase((size_t)n_seqs + 1, 0);
+    for (int64_t b = 0; b < n_seqs; b++) {
+        vbase[(size_t)b + 1] = vbase[(size_t)b] + (int64_t)pos[(size_t)b].size();
+        ebase[(size_t)b + 1] = ebase[(size_t)b] + (int64_t)wt[(size_t)b].size();
+    }
+    const int64_t nv = vbase[(size_t)n_seqs], ne = ebase[(size_t)n_seqs];
+    std::vector<int64_t> rowptr((size_t)(nv + n_seqs));
+    std::vector<int32_t> fpos((size_t)std::max<int64_t>(nv, 1)), fadj((size_t)std::max<int64_t>(2 * ne, 1)), fep(fadj.size());
+    std::vector<double> fwt((size_t)std::max<int64_t>(ne, 1));
+    parallel_for(n_seqs, [&](int64_t b) {
+        const size_t B = (size_t)b;
+        int64_t *rp = rowptr.data() + vbase[B] + b;
+        for (size_t x = 0; x < rows[B].size(); x++) rp[x] = 2 * ebase[B] + rows[B][x];
+        std::copy(pos[B].begin(), pos[B].end(), fpos.begin() + vbase[B]);
+        std::copy(adj[B].begin(), adj[B].end(), fadj.begin() + 2 * ebase[B]);
+        std::copy(ep[B].begin(), ep[B].end(), fep.begin() + 2 * ebase[B]);
+        std::copy(wt[B].begin(), wt[B].end(), fwt.begin() + ebase[B]);
+    });
+
+    // the three tiers, each longest first; a sequence without an edge has no pair and is not launched
+    const int smax = ed_smem_max_n(ctx->smem_optin);
+    std::vector<int32_t> ord[3];                      // global, CTA, warp
+    for (int64_t b = 0; b < n_seqs; b++) {
+        const int64_t n = offsets[b + 1] - offsets[b];
+        if (ebase[(size_t)b + 1] > ebase[(size_t)b]) ord[n > smax ? 0 : n > ED_WARP_MAX_N ? 1 : 2].push_back((int32_t)b);
+    }
+    auto longest_first = [&](int32_t a, int32_t c) { return offsets[a + 1] - offsets[a] > offsets[c + 1] - offsets[c]; };
+    std::vector<int32_t> order;
+    for (auto &o : ord) { std::stable_sort(o.begin(), o.end(), longest_first); order.insert(order.end(), o.begin(), o.end()); }
+
+    cudaStream_t st = ctx->stream;
+    int64_t *d_vb, *d_eb, *d_rowptr, *d_obase; int32_t *d_pos, *d_adj, *d_ep; double *d_wt, *d_maxw;
+    int32_t *d_order, *d_outp, *d_outn; int *d_cnt;
+    TRY(upload(ctx, ED_VBASE, vbase.data(), vbase.size(), &d_vb));
+    TRY(upload(ctx, ED_EBASE, ebase.data(), ebase.size(), &d_eb));
+    TRY(upload(ctx, ED_ROWPTR, rowptr.data(), rowptr.size(), &d_rowptr));
+    TRY(upload(ctx, ED_POS, fpos.data(), (size_t)nv, &d_pos));
+    TRY(upload(ctx, ED_ADJ, fadj.data(), (size_t)(2 * ne), &d_adj));
+    TRY(upload(ctx, ED_EP, fep.data(), (size_t)(2 * ne), &d_ep));
+    TRY(upload(ctx, ED_WT, fwt.data(), (size_t)ne, &d_wt));
+    TRY(upload(ctx, ED_MAXW, maxw.data(), maxw.size(), &d_maxw));
+    TRY(upload(ctx, ED_ORDER, order.data(), order.size(), &d_order));
+    TRY(upload(ctx, ED_OUTBASE, out_base.data(), (size_t)n_seqs, &d_obase));
+    TRY(dalloc(ctx, ED_OUTP, (size_t)(2 * cap), &d_outp));
+    TRY(dalloc(ctx, ED_OUTN, (size_t)n_seqs, &d_outn));
+    TRY(dalloc(ctx, ED_CNT, 3, &d_cnt));
+    CK(cudaMemsetAsync(d_outn, 0, (size_t)n_seqs * sizeof(int32_t), st));
+    CK(cudaMemsetAsync(d_cnt, 0, 3 * sizeof(int), st));
+    EdBatch eb{};
+    eb.vbase = d_vb; eb.ebase = d_eb; eb.rowptr = d_rowptr; eb.pos = d_pos; eb.adj = d_adj; eb.ep = d_ep;
+    eb.wt = d_wt; eb.maxw = d_maxw; eb.out_base = d_obase; eb.out_pairs = d_outp; eb.out_n = d_outn;
+
+    // launch geometry per tier: the node-state bytes a team needs (the most nodes of the tier), its slot (node state
+    // for the global tier, then the edge state of the tier's largest graph), the number of teams
+    struct Tier { int n = 0, grid = 0, teams_per_cta = 1; int64_t vbytes = 0, slot = 0; size_t smem = 0; };
+    Tier T3[3];
+    for (int t = 0; t < 3; t++) {
+        Tier &ti = T3[t];
+        ti.n = (int)ord[t].size();
+        if (!ti.n) continue;
+        int vmax = 0; int64_t ewords = 0;
+        for (const int32_t b : ord[t]) {
+            const int v = (int)(vbase[(size_t)b + 1] - vbase[(size_t)b]);
+            vmax = std::max(vmax, v);
+            ewords = std::max(ewords, ed_edge_words(v, ebase[(size_t)b + 1] - ebase[(size_t)b]));
+        }
+        ti.vbytes = (int64_t)ed_layout(vmax).total;
+        ti.slot = (t == 0 ? ti.vbytes : 0) + 4 * ewords;
+        int occ = 0;
+        if (t == 2) {
+            ti.teams_per_cta = ED_WPC;
+            ti.smem = ed_warp_smem(vmax);
+            CK(cudaFuncSetAttribute(k_edmonds<1, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)ti.smem));
+            CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_edmonds<1, true>, ED_WPC * 32, ti.smem));
+            ti.grid = (int)std::min<int64_t>((ti.n + ED_WPC - 1) / ED_WPC, (int64_t)ctx->sm_count * std::max(occ, 1));
+        } else if (t == 1) {
+            ti.smem = ed_cta_smem(vmax, true);
+            CK(cudaFuncSetAttribute(k_edmonds<ED_CTA_TW, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)ti.smem));
+            CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_edmonds<ED_CTA_TW, true>, ED_CTA_TW * 32, ti.smem));
+            ti.grid = (int)std::min<int64_t>((int64_t)ti.n, (int64_t)ctx->sm_count * std::max(occ, 1));
+        } else {
+            ti.smem = ed_cta_smem(0, false);
+            ti.grid = std::min(ti.n, ctx->sm_count);
+        }
+    }
+    // the cap: each tier gets a third of it, and at least one CTA
+    int64_t ws_bytes = 0, at[3];
+    for (int t = 0; t < 3; t++) {
+        Tier &ti = T3[t];
+        at[t] = ws_bytes;
+        if (!ti.n) continue;
+        const int64_t per_cta = ti.slot * ti.teams_per_cta;
+        ti.grid = (int)std::min<int64_t>(ti.grid, std::max<int64_t>(1, ED_WORKSPACE_CAP / 3 / per_cta));
+        ws_bytes += ((int64_t)ti.grid * per_cta + 255) & ~(int64_t)255;
+    }
+    if ((size_t)ws_bytes > ctx->ed_ws_bytes) {
+        if (ctx->ed_ws) cudaFree(ctx->ed_ws);
+        ctx->ed_ws = nullptr; ctx->ed_ws_bytes = 0;
+        CK(cudaMalloc(&ctx->ed_ws, (size_t)ws_bytes));
+        ctx->ed_ws_bytes = (size_t)ws_bytes;
+    }
+    unsigned char *ws = (unsigned char *)ctx->ed_ws;
+    const int ng = T3[0].n, nc = T3[1].n, nw = T3[2].n;
+    CK(cudaEventRecord(ctx->ev0, st));
+    CK(cudaEventRecord(ctx->ev_start, st));          // the uploads are done: where the second stream starts
+    if (nw) {                                         // warp tier, on the second stream
+        EdBatch w = eb;
+        w.n_items = nw; w.order = d_order + ng + nc; w.counter = d_cnt + 2; w.ws = ws + at[2]; w.slot_bytes = T3[2].slot;
+        CK(cudaStreamWaitEvent(ctx->s_k2, ctx->ev_start, 0));
+        k_edmonds<1, true><<<T3[2].grid, ED_WPC * 32, T3[2].smem, ctx->s_k2>>>(w, T3[2].vbytes);
+        CK(cudaGetLastError());
+        CK(cudaEventRecord(ctx->ev_k2done, ctx->s_k2));
+        ctx->n_launches++;
+    }
+    if (ng) {                                         // global tier
+        EdBatch g = eb;
+        g.n_items = ng; g.order = d_order; g.counter = d_cnt; g.ws = ws + at[0]; g.slot_bytes = T3[0].slot;
+        k_edmonds<ED_CTA_TW, false><<<T3[0].grid, ED_CTA_TW * 32, T3[0].smem, st>>>(g, T3[0].vbytes);
+        CK(cudaGetLastError());
+        ctx->n_launches++;
+    }
+    if (nc) {                                         // CTA tier
+        EdBatch c = eb;
+        c.n_items = nc; c.order = d_order + ng; c.counter = d_cnt + 1; c.ws = ws + at[1]; c.slot_bytes = T3[1].slot;
+        k_edmonds<ED_CTA_TW, true><<<T3[1].grid, ED_CTA_TW * 32, T3[1].smem, st>>>(c, T3[1].vbytes);
+        CK(cudaGetLastError());
+        ctx->n_launches++;
+    }
+    if (nw) CK(cudaStreamWaitEvent(st, ctx->ev_k2done, 0));
+    CK(cudaEventRecord(ctx->ev1, st));
+    std::vector<int32_t> outn((size_t)n_seqs);
+    CK(cudaMemcpyAsync(outn.data(), d_outn, (size_t)n_seqs * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+    if (cap > 0) CK(cudaMemcpyAsync(pairs, d_outp, (size_t)(2 * cap) * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+    CK(cudaStreamSynchronize(st));
+    float ms = 0.f;
+    if (cudaEventElapsedTime(&ms, ctx->ev0, ctx->ev1) == cudaSuccess) ctx->kernel_ms = ms;
+    for (int64_t b = 0; b < n_seqs; b++)
+        if (outn[(size_t)b] < 0) {
+            ctx->err = "edmonds: sequence " + std::to_string(b) + ": internal capacity exceeded";
+            return SQRN_E_UNSUPPORTED;
+        }
+    // sequence b's pairs were written at out_base[b] in node order: sort them by v, then pack them in sequence order
+    // (in place: never moves right)
+    parallel_for(n_seqs, [&](int64_t b) {
+        int32_t *p = pairs + 2 * out_base[(size_t)b];
+        std::vector<std::pair<int32_t, int32_t>> pr((size_t)outn[(size_t)b]);
+        for (size_t k = 0; k < pr.size(); k++) pr[k] = {p[2 * k], p[2 * k + 1]};
+        std::sort(pr.begin(), pr.end());
+        for (size_t k = 0; k < pr.size(); k++) { p[2 * k] = pr[k].first; p[2 * k + 1] = pr[k].second; }
+    });
+    int64_t atp = 0;
+    for (int64_t b = 0; b < n_seqs; b++) {
+        pair_offsets[b] = atp;
+        const int64_t m = outn[(size_t)b];
+        if (m && atp != out_base[(size_t)b]) memmove(pairs + 2 * atp, pairs + 2 * out_base[(size_t)b], (size_t)m * 2 * sizeof(int32_t));
+        atp += m;
+    }
+    pair_offsets[n_seqs] = atp;
+    if (cap > atp) memset(pairs + 2 * atp, 0, (size_t)(cap - atp) * 2 * sizeof(int32_t));     // (no stale device memory)
+    return SQRN_OK;
+}
+
+extern "C" int sqrn_edmonds_batch(sqrn_ctx *ctx, int64_t n_seqs, const int64_t *offsets, const int64_t *stem_offsets,
+                                  const int32_t *stems, const double *scores, double power, int64_t *pair_offsets,
+                                  int32_t *pairs)
+{
+    return guarded(ctx, [&] { return sqrn_edmonds_batch_impl(ctx, n_seqs, offsets, stem_offsets, stems, scores, power, pair_offsets, pairs); });
 }
